@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config small] [--batch 32] [--dtype fp16]
     python bench.py --impl reference ...      # the unmodified reference's CPU forward (baseline/_ref) on the host cores
+    python bench.py --dump-outputs DIR ...    # also write the last timed step's predictions as DIR/<name>.npy
     torchrun --nproc-per-node N bench.py --gpus N ...   # one process per GPU, image-sharded replicas
 
 One "step" = one forward pass of `batch` synthetic 640x640 images per GPU through the C-ABI engine
@@ -9,6 +10,11 @@ One "step" = one forward pass of `batch` synthetic 640x640 images per GPU throug
 with the inputs resident in HBM; `e2e` = the same through the public nn.Module call with PINNED HOST
 inputs (H2D of every batch and D2H of the predictions inside the timed region, double buffered).
 Rank 0 prints ONE JSON line.
+
+With --dump-outputs DIR rank 0 writes what the last timed step returned to its caller, pred_logits [batch, queries,
+classes] and pred_boxes [batch, queries, 4], as float32 DIR/pred_logits.npy and DIR/pred_boxes.npy.  Weights and inputs
+are seeded, so two builds run with the same arguments can be compared output for output.  When the two arrays would
+exceed 64 MB, a fixed seeded sample of the images is written instead, with its image indices in DIR/image_index.npy.
 """
 import argparse
 import json
@@ -25,6 +31,7 @@ sys.path.insert(0, os.path.join(ROOT, "lw-detr_b200"))
 
 import torch  # noqa: E402
 
+DUMP_LIMIT_BYTES = 63_000_000        # --dump-outputs stays under 64 MB, .npy headers and the image index included
 DEFAULT_BATCH = {"tiny": 32, "small": 32, "medium": 64, "large": 32, "xlarge": 16}
 FLOPS_PER_IMAGE = {"tiny": 21.40e9, "small": 31.76e9, "medium": 83.93e9, "large": 137.51e9, "xlarge": 342.51e9}  # SURVEY.md 8
 
@@ -178,7 +185,12 @@ def main():
     ap.add_argument("--profile-out", default=None, help="write the per-op timing table (JSON) here")
     ap.add_argument("--no-per-config", action="store_true", help="skip the per_config block (the other four BASELINE configs, N = 1 only)")
     ap.add_argument("--e2e-input", default="uint8", choices=["uint8", "fp32"], help="what the end-to-end arm holds on the host")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write the last timed step's predictions to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -217,7 +229,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     r = measure_config(cfg_name, batch, dtype_name, a.steps, warmup, dev, rank, world, local, graph=not a.no_graph, pdl=not a.no_pdl,
-                       profile_out=a.profile_out, clocks=True, e2e_input=a.e2e_input)
+                       profile_out=a.profile_out, clocks=True, e2e_input=a.e2e_input, dump_dir=a.dump_outputs if rank == 0 else None)
 
     cpu = None
     if rank == 0 and world == 1:
@@ -263,10 +275,27 @@ def main():
         dist.destroy_process_group()
 
 
+def dump_outputs(out, dump_dir):
+    """Writes the predictions of one step as float32 .npy files (see the module docstring)."""
+    import numpy as np
+    arrays = {k: out[k].detach().float().cpu() for k in ("pred_logits", "pred_boxes")}
+    batch = arrays["pred_logits"].shape[0]
+    per_image = sum(v[0].numel() * 4 for v in arrays.values())
+    keep = min(batch, DUMP_LIMIT_BYTES // (per_image + 8))
+    os.makedirs(dump_dir, exist_ok=True)
+    if keep < batch:
+        idx = torch.randperm(batch, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["image_index"] = idx.double()
+    for k, v in arrays.items():
+        np.save(os.path.join(dump_dir, k + ".npy"), v.numpy())
+
+
 def measure_config(cfg_name, batch, dtype_name, steps, warmup, dev, rank, world, local, graph=True, pdl=True, profile_out=None, clocks=True,
-                   e2e_input="uint8"):
+                   e2e_input="uint8", dump_dir=None):
     """One LW-DETR configuration on this rank's GPU: device-resident throughput, end-to-end throughput through the public
-    module call with host inputs, batch-1 latencies and the per-kernel table.  Returns a dict (see main)."""
+    module call with host inputs, batch-1 latencies and the per-kernel table.  Returns a dict (see main).  With dump_dir the
+    predictions of the last timed step are written there (dump_outputs)."""
     import torch.distributed as dist
     from b200.config import CONFIGS
     from b200.synth import synth_images, synth_state_dict
@@ -316,7 +345,10 @@ def measure_config(cfg_name, batch, dtype_name, steps, warmup, dev, rank, world,
         barrier()
         return ms.item()
 
-    dev_step = lambda i: eng.forward(xs[i & 1], want_aux=False)
+    last = {}
+
+    def dev_step(i):
+        last["out"] = eng.forward(xs[i & 1], want_aux=False)
     for i in range(warmup):
         dev_step(i)
     sampler = ClockSampler(local)
@@ -326,6 +358,8 @@ def measure_config(cfg_name, batch, dtype_name, steps, warmup, dev, rank, world,
     load_t0 = time.time()
     ms_total = timed(dev_step, steps)
     load_t1 = time.time()
+    if dump_dir:
+        dump_outputs(last["out"], dump_dir)       # before any untimed step below replaces it
     if rank == 0 and clocks:
         # a short timed region can fall between two 100 ms nvidia-smi samples: keep the same step running
         # (untimed) until at least three samples were taken under this load

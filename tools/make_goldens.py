@@ -85,6 +85,68 @@ def make_padded_golden():
     print("padded", out["pred_logits"].shape)
 
 
+def make_live_goldens():
+    """What the tests used to compute by running the reference next to them, stored so that they need no reference tree:
+      ref_tiny_seed5.npz   the tiny forward on weight seed 5: dict outputs on two images (image seed 9), and on the first
+                           image alone the dict outputs and the forward_export tuple after LWDETR.export()
+      ref_msda_checker.npz models/ops/test.py's inputs (torch.manual_seed(3), double then float pass) and the output of
+                           its checker ms_deform_attn_core_pytorch on them
+      demo_small_args.json the namespace demo/demo.py's argument parser yields for the LW-DETR-small evaluation flags"""
+    cfg = CONFIGS["tiny"]
+    model, _, _ = ref_import.build_reference(cfg)
+    model.load_state_dict(synth_state_dict(cfg, 5), strict=True)
+    x1 = synth_images(1, 9)
+    with torch.no_grad():
+        two = model(synth_images(2, 9))
+        one = model(x1)
+        model.export()
+        boxes, logits = model(x1)
+    np.savez_compressed(os.path.join(GOLD, "ref_tiny_seed5.npz"), pred_logits=two["pred_logits"].numpy(),
+                        pred_boxes=two["pred_boxes"].numpy(), one_pred_logits=one["pred_logits"].numpy(),
+                        one_pred_boxes=one["pred_boxes"].numpy(), export_boxes=boxes.numpy(), export_logits=logits.numpy(),
+                        meta=np.array([2, 5, 9], dtype=np.int64))
+
+    ref_import._install_shims()
+    ops = os.path.join(ref_import.REF, "models", "ops")
+    sys.path.insert(0, ops)
+    try:
+        from functions.ms_deform_attn_func import ms_deform_attn_core_pytorch as core
+    finally:
+        sys.path.remove(ops)
+    N, M, D, Lq, L, P = 1, 2, 2, 2, 2, 2                                   # models/ops/test.py:27-31
+    shapes = torch.as_tensor([(6, 4), (3, 2)], dtype=torch.long)
+    S = int(shapes.prod(1).sum())
+    torch.manual_seed(3)
+    rec = {"shapes": shapes.numpy()}
+    for i, cast in enumerate((lambda t: t.double(), lambda t: t)):
+        value = torch.rand(N, S, M, D) * 0.01
+        loc = torch.rand(N, Lq, M, L, P, 2)
+        aw = torch.rand(N, Lq, M, L, P) + 1e-5
+        aw /= aw.sum(-1, keepdim=True).sum(-2, keepdim=True)
+        rec.update({"value%d" % i: value.numpy(), "loc%d" % i: loc.numpy(), "aw%d" % i: aw.numpy(),
+                    "out%d" % i: core(cast(value).permute(0, 2, 3, 1), shapes, cast(loc), cast(aw)).numpy()})
+    np.savez_compressed(os.path.join(GOLD, "ref_msda_checker.npz"), **rec)
+
+    import importlib.util
+    sys.path.insert(0, ref_import.REF)
+    try:
+        spec = importlib.util.spec_from_file_location("ref_demo", os.path.join(ref_import.REF, "demo", "demo.py"))
+        demo = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(demo)
+        ns = demo.get_args_parser().parse_args(DEMO_SMALL_FLAGS + ["--weights", "-", "--input", "-"])
+    finally:
+        sys.path.remove(ref_import.REF)
+    args = {k: v for k, v in vars(ns).items() if k not in ("weights", "input", "output_dir", "device")}
+    with open(os.path.join(GOLD, "demo_small_args.json"), "w") as f:
+        json.dump(args, f, indent=0, sort_keys=True)
+    print("live goldens: tiny seed 5, MSDA checker, demo args (%d fields)" % len(args))
+
+
+DEMO_SMALL_FLAGS = ("--encoder vit_tiny --vit_encoder_num_layers 10 --window_block_indexes 0 1 3 6 7 9 --out_feature_indexes 2 4 5 9 "
+                    "--projector_scale P4 --hidden_dim 256 --sa_nheads 8 --ca_nheads 16 --dec_n_points 2 --dec_layers 3 --group_detr 13 "
+                    "--two_stage --bbox_reparam --lite_refpoint_refine --num_select 300").split()     # scripts/lwdetr_small_coco_eval.sh:10-24
+
+
 def main():
     torch.set_num_threads(os.cpu_count())
     os.makedirs(GOLD, exist_ok=True)
@@ -93,6 +155,9 @@ def main():
         return
     if "--padded-only" in sys.argv:
         make_padded_golden()
+        return
+    if "--live-only" in sys.argv:
+        make_live_goldens()
         return
     for name, B in CASES:
         cfg = CONFIGS[name]
@@ -132,6 +197,7 @@ def main():
         print(name, "B=%d" % B, {k: v.shape for k, v in rec.items() if k.startswith("pred")})
     make_postprocess_goldens()
     make_padded_golden()
+    make_live_goldens()
 
 
 if __name__ == "__main__":
