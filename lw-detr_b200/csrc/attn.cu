@@ -8,17 +8,16 @@
 // dimension and a per-head column offset, so the packed qkv GEMM output is consumed in place.
 //
 // Kernels in this file (register-resident flash attention: mma.sync m16n8k16 with fp32 accumulation, K/V chunks
-// in a 3-stage cp.async ring, exp2 against the running maximum of the raw scores):
-//   attn_kernel       - sequences longer than 112 tokens: global attention at head dim 16, decoder self-attention
-//   attn_short_kernel - the 100-token windows, persistent CTAs walking (window, head) items
-// Long packed-qkv sequences at head dim >= 32 are dispatched to the tcgen05 kernel in attn_tc.cu instead
-// (attention_launch below; measured crossover in DESIGN.md 3.1).
+// in a 3-stage cp.async ring, exp2 against the running maximum of the raw scores) take what the tcgen05 kernels do not:
+//   attn_kernel       - sequences longer than 112 tokens (decoder self-attention)
+//   attn_short_kernel - sequences of up to 112 tokens, persistent CTAs walking (window, head) items
+// Packed qkv at head dims 16 and 32 goes to the slot kernel (attn_slots.cu), long packed sequences at head dim 64 to
+// attn_tc.cu (attention_launch below; measured crossovers in DESIGN.md 3.1).
 #include "attn.h"
 #include "launch.h"
 #include "ptx.cuh"
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace lwb {
 
@@ -58,11 +57,6 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N> __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
-__device__ __forceinline__ float fast_exp2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
 
 static constexpr int KC = 64;      // keys per shared-memory chunk
 static constexpr int NSTAGE = 3;   // K/V ring: chunk ch+2 is prefetched while ch is consumed -> one barrier per chunk
@@ -70,13 +64,11 @@ static constexpr int NSTAGE = 3;   // K/V ring: chunk ch+2 is prefetched while c
 // One 64-key chunk of the online-softmax attention for a warp's 16 query rows.
 //   qf: Q fragments (A operand); cK / cV: the chunk's K and V rows in shared memory ([64][LDS]);
 //   kbase: index of the chunk's first key; keys >= seqlen are masked.
-//   PM: bit nt set = the exponentials of n-tile nt take the polynomial exp2 on the FMA pipe (ptx.cuh) instead of the MUFU.
 //   NT: 8-key n-tiles of this chunk that can hold valid keys (8 = the full 64-key chunk; the second chunk of a 100-token
 //       window only needs 5: no scores, exponentials or P V steps are spent on keys that cannot exist).
-template <typename T, int DH, uint32_t PM = 0, int NT = 8>
+template <typename T, int DH, int NT = 8>
 __device__ __forceinline__ void attn_chunk(const uint32_t (&qf)[DH / 16][4], const T* cK, const T* cV, int kbase, int seqlen,
-                                           float scale_log2, float inv_scale_log2, int lane, float (&m_run)[2], float (&lsum)[4],
-                                           float (&o)[DH / 8][4]) {
+                                           float scale_log2, int lane, float (&m_run)[2], float (&lsum)[4], float (&o)[DH / 8][4]) {
   constexpr int LDS = DH + 8;
   const int t4 = lane & 3;
   const uint32_t ones2 = Cvt<T>::pack(1.f, 1.f);
@@ -120,12 +112,11 @@ __device__ __forceinline__ void attn_chunk(const uint32_t (&qf)[DH / 16][4], con
       mx[h] = fmaxf(mx[h], __shfl_xor_sync(0xffffffffu, mx[h], 1));
       mx[h] = fmaxf(mx[h], __shfl_xor_sync(0xffffffffu, mx[h], 2));
       const float m_new = fmaxf(m_run[h], mx[h]);            // running max of the RAW scores
-      alpha[h] = fast_exp2((m_run[h] - m_new) * scale_log2);
+      alpha[h] = ex2((m_run[h] - m_new) * scale_log2);
       m_run[h] = m_new;
       msc[h] = m_new * scale_log2;
     }
     uint32_t pf[NTP / 2][4];
-    const uint64_t c2 = f2_pack(scale_log2, scale_log2);
 #pragma unroll
     for (int nt = 0; nt < NTP; ++nt) {
       if (nt >= NT) {                                          // padding half of the last 16-key step
@@ -133,17 +124,10 @@ __device__ __forceinline__ void attn_chunk(const uint32_t (&qf)[DH / 16][4], con
         pf[nt >> 1][(nt & 1) * 2 + 1] = 0u;
         continue;
       }
-      float p0, p1, p2, p3;
-      if ((PM >> nt) & 1u) {
-        constexpr float kMagic = 12582912.f;
-        exp2_poly2(s[nt][0], s[nt][1], m_run[0] - 125.f * inv_scale_log2, c2, f2_pack(kMagic - msc[0], kMagic - msc[0]), f2_pack(-msc[0], -msc[0]), p0, p1);
-        exp2_poly2(s[nt][2], s[nt][3], m_run[1] - 125.f * inv_scale_log2, c2, f2_pack(kMagic - msc[1], kMagic - msc[1]), f2_pack(-msc[1], -msc[1]), p2, p3);
-      } else {
-        p0 = fast_exp2(fmaf(s[nt][0], scale_log2, -msc[0]));
-        p1 = fast_exp2(fmaf(s[nt][1], scale_log2, -msc[0]));
-        p2 = fast_exp2(fmaf(s[nt][2], scale_log2, -msc[1]));
-        p3 = fast_exp2(fmaf(s[nt][3], scale_log2, -msc[1]));
-      }
+      const float p0 = ex2(fmaf(s[nt][0], scale_log2, -msc[0]));
+      const float p1 = ex2(fmaf(s[nt][1], scale_log2, -msc[0]));
+      const float p2 = ex2(fmaf(s[nt][2], scale_log2, -msc[1]));
+      const float p3 = ex2(fmaf(s[nt][3], scale_log2, -msc[1]));
       // C fragments of n-tiles (2j, 2j+1) form the A fragment of key-step j
       pf[nt >> 1][(nt & 1) * 2 + 0] = Cvt<T>::pack(p0, p1);
       pf[nt >> 1][(nt & 1) * 2 + 1] = Cvt<T>::pack(p2, p3);
@@ -174,7 +158,7 @@ __device__ __forceinline__ void attn_chunk(const uint32_t (&qf)[DH / 16][4], con
     }
 }
 
-template <typename T, int DH, int WARPS, uint32_t PM = 0>
+template <typename T, int DH, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32) attn_kernel(const AttnArgs p) {
   pdl_sync();   // programmatic dependent launch: release the successor, wait for the predecessor (launch.h)
   constexpr int QROWS = WARPS * 16;
@@ -242,7 +226,7 @@ __global__ void __launch_bounds__(WARPS * 32) attn_kernel(const AttnArgs p) {
     const T* cK = sK + buf * KC * LDS;
     const T* cV = sV + buf * KC * LDS;
 
-    attn_chunk<T, DH, PM>(qf, cK, cV, ch * KC, p.seqlen, p.scale_log2, 1.f / p.scale_log2, lane, m_run, lsum, o);
+    attn_chunk<T, DH>(qf, cK, cV, ch * KC, p.seqlen, p.scale_log2, lane, m_run, lsum, o);
   }
 
   // ---- finalise: divide by the row sums, stage through this warp's Q rows, 16-byte coalesced stores
@@ -271,7 +255,7 @@ __global__ void __launch_bounds__(WARPS * 32) attn_kernel(const AttnArgs p) {
 // running at the same time read neighbouring 32..128-byte slices of the same token rows) and prefetch item
 // i+2 into a 3-deep buffer ring while item i is computed - the HBM latency is hidden behind the math and the
 // kernel runs at the larger of its HBM time and its exp (MUFU) time.
-template <typename T, int DH, uint32_t PM = 0>
+template <typename T, int DH>
 __global__ void __launch_bounds__(7 * 32) attn_short_kernel(const AttnArgs p) {
   pdl_sync();   // programmatic dependent launch: release the successor, wait for the predecessor (launch.h)
   constexpr int WARPS = 7, QROWS = 112, KROWS = 128, NBUF = 3;
@@ -330,10 +314,9 @@ __global__ void __launch_bounds__(7 * 32) attn_short_kernel(const AttnArgs p) {
     for (int i = 0; i < DH / 8; ++i) o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f;
     float m_run[2] = {-INFINITY, -INFINITY};
     float lsum[4] = {0.f, 0.f, 0.f, 0.f};
-    const float inv_c = 1.f / p.scale_log2;
-    attn_chunk<T, DH, PM>(qf, sK, sV, 0, p.seqlen, p.scale_log2, inv_c, lane, m_run, lsum, o);
-    if (p.seqlen > KC + 40) attn_chunk<T, DH, PM, 6>(qf, sK + KC * LDS, sV + KC * LDS, KC, p.seqlen, p.scale_log2, inv_c, lane, m_run, lsum, o);   // keys 64..111 (seqlen <= 112 here)
-    else if (p.seqlen > KC) attn_chunk<T, DH, PM, 5>(qf, sK + KC * LDS, sV + KC * LDS, KC, p.seqlen, p.scale_log2, inv_c, lane, m_run, lsum, o);   // keys 64..103: the 100-token windows
+    attn_chunk<T, DH>(qf, sK, sV, 0, p.seqlen, p.scale_log2, lane, m_run, lsum, o);
+    if (p.seqlen > KC + 40) attn_chunk<T, DH, 6>(qf, sK + KC * LDS, sV + KC * LDS, KC, p.seqlen, p.scale_log2, lane, m_run, lsum, o);   // keys 64..111 (seqlen <= 112 here)
+    else if (p.seqlen > KC) attn_chunk<T, DH, 5>(qf, sK + KC * LDS, sV + KC * LDS, KC, p.seqlen, p.scale_log2, lane, m_run, lsum, o);   // keys 64..103: the 100-token windows
 
     const float l_run[2] = {1.f / lsum[0], 1.f / lsum[2]};
     T* sO = sQ + warp * 16 * LDS;          // this warp's own Q rows: already consumed into qf
@@ -356,60 +339,44 @@ __global__ void __launch_bounds__(7 * 32) attn_short_kernel(const AttnArgs p) {
   }
 }
 
-template <typename T, int DH, uint32_t PM = 0>
+template <typename T, int DH>
 static int launch_short(const AttnArgs& a, cudaStream_t st) {
   constexpr int LDS = DH + 8;
   const size_t smem = static_cast<size_t>(3) * (112 + 256) * LDS * sizeof(T);
-  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_short_kernel<T, DH, PM>), 200 * 1024)) return e;
+  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_short_kernel<T, DH>), 200 * 1024)) return e;
   static int ctas_per_sm = 0;   // a property of the kernel image and the sm_100a SM, identical on every device of a B200 box
   if (!ctas_per_sm) {
     int n = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, attn_short_kernel<T, DH, PM>, 7 * 32, smem);
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, attn_short_kernel<T, DH>, 7 * 32, smem);
     if (e != cudaSuccess) return static_cast<int>(e);
     ctas_per_sm = n > 0 ? n : 1;
   }
   const int sms = current_device_sms();
   const long long items = static_cast<long long>(a.nseq) * a.heads;
   const unsigned grid = static_cast<unsigned>(std::min<long long>(items, static_cast<long long>(sms) * ctas_per_sm));
-  launch_k(attn_short_kernel<T, DH, PM>, dim3(grid), dim3(7 * 32), smem, st, a);
+  launch_k(attn_short_kernel<T, DH>, dim3(grid), dim3(7 * 32), smem, st, a);
   return static_cast<int>(cudaGetLastError());
 }
 
-template <typename T, int DH, int WARPS, uint32_t PM = 0>
+template <typename T, int DH, int WARPS>
 static int launch(const AttnArgs& a, cudaStream_t st) {
   constexpr int LDS = DH + 8;
   const size_t smem = static_cast<size_t>(WARPS * 16 + 2 * NSTAGE * KC) * LDS * sizeof(T);
-  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_kernel<T, DH, WARPS, PM>), 96 * 1024)) return e;
+  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_kernel<T, DH, WARPS>), 96 * 1024)) return e;
   dim3 grid((a.seqlen + WARPS * 16 - 1) / (WARPS * 16), a.heads, a.nseq);
-  launch_k(attn_kernel<T, DH, WARPS, PM>, dim3(grid), dim3(WARPS * 32), smem, st, a);
+  launch_k(attn_kernel<T, DH, WARPS>, dim3(grid), dim3(WARPS * 32), smem, st, a);
   return static_cast<int>(cudaGetLastError());
-}
-
-// Share of the exponentials that takes the polynomial exp2 (FMA pipe) instead of the MUFU in the mma.sync kernels at
-// head dims 16 / 32, where the MUFU is the roof: 0 = none, 1 = 2 of 8 n-tiles, 2 = 3 of 8.  LWDETR_B200_ATTN_POLY
-// overrides the default for A/B measurements.
-static int poly_policy() {
-  static int v = [] {
-    const char* e = getenv("LWDETR_B200_ATTN_POLY");
-    return e ? atoi(e) : 0;
-  }();
-  return v;
 }
 
 template <typename T>
 static int dispatch(const AttnArgs& a, int dh, cudaStream_t st) {
-  const int pol = poly_policy();
   if (a.seqlen <= 112) {
-    if (dh == 16) return pol == 1 ? launch_short<T, 16, 0x24u>(a, st) : pol == 2 ? launch_short<T, 16, 0x49u>(a, st) : launch_short<T, 16>(a, st);
-    if (dh == 32) return pol == 1 ? launch_short<T, 32, 0x24u>(a, st) : pol == 2 ? launch_short<T, 32, 0x49u>(a, st) : launch_short<T, 32>(a, st);
+    if (dh == 16) return launch_short<T, 16>(a, st);
+    if (dh == 32) return launch_short<T, 32>(a, st);
     if (dh == 64) return launch_short<T, 64>(a, st);
     return -2;
   }
   const int warps = a.seqlen >= 1024 ? 8 : 4;
-  if (warps == 8 && pol > 0) {
-    if (dh == 16) return pol == 1 ? launch<T, 16, 8, 0x24u>(a, st) : launch<T, 16, 8, 0x49u>(a, st);
-    if (dh == 32) return pol == 1 ? launch<T, 32, 8, 0x24u>(a, st) : launch<T, 32, 8, 0x49u>(a, st);
-  }
 #define LWB_ATTN_CASE(D, W) if (dh == D && warps == W) return launch<T, D, W>(a, st);
   LWB_ATTN_CASE(16, 8) LWB_ATTN_CASE(16, 4)
   LWB_ATTN_CASE(32, 8) LWB_ATTN_CASE(32, 4)
@@ -421,40 +388,16 @@ static int dispatch(const AttnArgs& a, int dh, cudaStream_t st) {
 int attention_tc_launch(int dtype, const AttnArgs& a, int dh, int C, cudaStream_t st);      // attn_tc.cu
 int attention_slots_launch(int dtype, const AttnArgs& a, int dh, int C, cudaStream_t st);   // attn_slots.cu
 
-// Slot kernel (attn_slots.cu: tcgen05, one thread per row, partly polynomial exp2) for packed qkv:
-//   0 = never, 1 = head dim 16 always + head dim 32 for sequences of <= 128 tokens (the ViT windows),
-//   2 (default) = head dim 32 for every sequence length as well (global attention, B200, isolated: medium B=64 612 us against
-//   825 us of the attn_tc.cu kernel, large B=32 334 against 424).  Environment override for A/B measurements only.
-static int slots_policy() {
-  static int v = [] {
-    const char* e = getenv("LWDETR_B200_ATTN_SLOTS");
-    return e ? atoi(e) : 2;
-  }();
-  return v;
-}
-
-// 0 = mma.sync flash kernel everywhere, 1 = tcgen05 kernel for long packed-qkv sequences with dh >= 32 (default; measured
-// 18-22 % faster there, 10 % slower at dh = 16 where the mma.sync kernel's 6 warps per scheduler hide latency better),
-// 2 = tcgen05 kernel for every long packed-qkv sequence.  Environment override for A/B measurements only.
-static int tc_policy() {
-  static int v = [] {
-    const char* e = getenv("LWDETR_B200_ATTN_TC");
-    return e ? atoi(e) : 1;
-  }();
-  return v;
-}
-
+// Packed qkv at head dims 16 and 32 -> the slot kernel (attn_slots.cu; B200, isolated, global attention: medium B=64 612 us
+// against 825 us of the attn_tc.cu kernel, large B=32 334 against 424).  Long packed sequences at head dim 64 -> attn_tc.cu
+// (measured 18-22 % faster than the mma.sync kernel there).  Everything else -> the mma.sync kernels above.
 int attention_launch(int dtype, const AttnArgs& a, int dh, cudaStream_t st) {
   const long long dk = (static_cast<const char*>(a.k) - static_cast<const char*>(a.q)) / 2;
   const long long dv = (static_cast<const char*>(a.v) - static_cast<const char*>(a.q)) / 2;
   const bool packed = dk > 0 && dv == 2 * dk && a.ldq == a.ldk && a.ldq == a.ldv && dk == static_cast<long long>(a.heads) * dh &&
                       a.ldq >= 3 * dk && (reinterpret_cast<uintptr_t>(a.q) & 15) == 0;
-  const int sp = slots_policy();
-  if (packed && sp > 0 && (dh == 16 || (dh == 32 && (a.seqlen <= 128 || sp >= 2))))
-    return attention_slots_launch(dtype, a, dh, static_cast<int>(dk), st);
-  const int pol = tc_policy();
-  if (packed && a.seqlen >= 512 && (pol == 2 || (pol == 1 && dh >= 32)))
-    return attention_tc_launch(dtype, a, dh, static_cast<int>(dk), st);
+  if (packed && (dh == 16 || dh == 32)) return attention_slots_launch(dtype, a, dh, static_cast<int>(dk), st);
+  if (packed && a.seqlen >= 512 && dh == 64) return attention_tc_launch(dtype, a, dh, static_cast<int>(dk), st);
   return dtype == DT_BF16 ? dispatch<__nv_bfloat16>(a, dh, st) : dispatch<__half>(a, dh, st);
 }
 

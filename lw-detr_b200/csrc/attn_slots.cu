@@ -14,20 +14,15 @@
 //                  without blocking) and the commits.  This lone thread is the slot's critical path (one dependent
 //                  instruction per 10-20 clocks): everything it does per chunk is incremental.
 //   * row sums out of the P V product (head dim 16): the B operand is [V | 1] with N = 32, the block of ones reached through
-//     the descriptor's leading byte offset (FUSED).
-//   * exp2: packed fp32x2 FMAs (fma.rn.f32x2) fold scale and max-subtraction.  A degree-3 polynomial exp2 on the FMA pipe
-//     (Cody-Waite split by the 1.5*2^23 magic add, max relative error 7.5e-5) can take PMASK/8 of the pairs; measured in
-//     the kernel it does not pay (the softmax threads are issue-bound before the two pipes overlap), so the default is 0.
+//     the descriptor's leading byte offset.
+//   * exp2: packed fp32x2 FMAs (fma.rn.f32x2) fold scale and max-subtraction, every exponential on the MUFU.
 //   * setmaxnreg moves registers from the driver warps (96 -> 64) to the softmax warps (96 -> 104), which hold a 64-score row
 //     chunk.  The pool is per CTA: what the 16 softmax warps take (16*32*8) must not exceed what the 4 driver warps release.
 //
-// Work decompositions (templates SHARED / LONG):
-//   independent slots (default): every slot walks its own (sequence, head, query tile) items with its own K/V ring;
-//   SHARED = lock step: the four slots of a CTA take consecutive query tiles of ONE (sequence, head) over ONE K/V ring
-//            (fills round-robin over the four drivers);
-//   LONG   = sequences of more than one tile (1600 tokens): warps whose rows lie beyond the sequence only keep the barrier
-//            protocol going; one-tile sequences (the 100-token windows) instead defer an item's epilogue into the next
-//            item's first chunk, and their tail chunk only exponentiates the valid keys (104 instead of 128).
+// Work decomposition: every slot walks its own (sequence, head, query tile) items with its own K/V ring.  LONG (template,
+// chosen from the sequence length) = sequences of more than one tile (1600 tokens): warps whose rows lie beyond the sequence
+// only keep the barrier protocol going; one-tile sequences (the 100-token windows) instead defer an item's epilogue into
+// the next item's first chunk, and their tail chunk only exponentiates the valid keys (104 instead of 128).
 // CTAs are persistent and walk their items with a fixed stride.
 #include "attn.h"
 #include "launch.h"
@@ -50,112 +45,9 @@ static constexpr int BK = 64;                  // keys per chunk
 static constexpr int W_DRIVER = 4 * SLOTS;      // warps 0-15: softmax (slot = warp / 4, TMEM lane quarter = warp % 4); 16-19: one driver per slot
 static constexpr int THREADS = 32 * (W_DRIVER + SLOTS);
 static constexpr float LAZY_LOG2 = 8.f;        // the row reference maximum moves only when exceeded by more than 2^8
-static constexpr float MAGIC = 12582912.f;     // 1.5 * 2^23
 
-__device__ __forceinline__ uint64_t desc(uint32_t smem_addr, uint32_t sbo_bytes, uint32_t layout_type) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(layout_type) << 61;
-  return d;
-}
-// same with an explicit leading byte offset: for an MN-major operand that is the distance between two 16-element
-// (32-byte) atoms along N - used to append a constant block of ones to the V tile (fused row sums, see FUSED below)
-__device__ __forceinline__ uint64_t desc_lbo(uint32_t smem_addr, uint32_t sbo_bytes, uint32_t layout_type, uint32_t lbo_bytes) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
-  d |= static_cast<uint64_t>((lbo_bytes >> 4) & 0x3FFFu) << 16;
-  d |= static_cast<uint64_t>((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(layout_type) << 61;
-  return d;
-}
-// D[tmem] (+)= A[tmem] * B[smem desc]
-__device__ __forceinline__ void mma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void ld_x32(uint32_t taddr, float* v) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,"
-      "%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-        "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-        "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void st_x16(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float ex2(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ uint64_t pk2(float a, float b) {
-  uint64_t r;
-  asm("mov.b64 %0, {%1,%2};" : "=l"(r) : "f"(a), "f"(b));
-  return r;
-}
-__device__ __forceinline__ void upk2(uint64_t v, float& a, float& b) { asm("mov.b64 {%0,%1}, %2;" : "=f"(a), "=f"(b) : "l"(v)); }
-__device__ __forceinline__ uint64_t fma2(uint64_t a, uint64_t b, uint64_t c) {
-  uint64_t d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  return d;
-}
-__device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
 template <int N> __device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
 template <int N> __device__ __forceinline__ void reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
-
-// 2^(s*c - m) for a pair without the MUFU: t = round(s*c - m) + MAGIC by one FFMA2, fraction f = s*c - m - round(..) in
-// [-0.5, 0.5] by a second one, degree-3 polynomial for 2^f, exponent added as an integer.  The raw scores are clamped at
-// smin = m - 125/c first: below that 2^x is 0 for every purpose here, and an unclamped argument would leave f outside the
-// polynomial's range - where it has a root, i.e. an exponent field that wraps into a huge value when the integer is added.
-__device__ __forceinline__ void exp2_poly_pair(float s0, float s1, float smin, uint64_t c2, uint64_t magic_minus_m2, uint64_t negm2, float& e0,
-                                               float& e1) {
-  const uint64_t s2 = pk2(fmaxf(s0, smin), fmaxf(s1, smin));
-  const uint64_t t2 = fma2(s2, c2, magic_minus_m2);
-  const uint64_t r2 = add2(t2, pk2(-MAGIC, -MAGIC));
-  const uint64_t u2 = fma2(r2, pk2(-1.f, -1.f), negm2);
-  const uint64_t f2 = fma2(s2, c2, u2);
-  uint64_t p2 = fma2(f2, pk2(0.05517164617776871f, 0.05517164617776871f), pk2(0.2426111251115799f, 0.2426111251115799f));
-  p2 = fma2(p2, f2, pk2(0.6932609677314758f, 0.6932609677314758f));
-  p2 = fma2(p2, f2, pk2(0.9999280571937561f, 0.9999280571937561f));
-  float p0, p1, t0, t1;
-  upk2(p2, p0, p1);
-  upk2(t2, t0, t1);
-  e0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
-  e1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
-}
 
 // Debug aid (LWDETR_B200_DEBUG_WAIT=1): barrier waits time out after ~50 ms and leave a record (source line, CTA, warp,
 // parity) in MAPPED HOST memory before trapping - readable after the device fault, see attention_slots_debug_dump().
@@ -232,17 +124,16 @@ struct SlotArgs {
   void* o;
   int ldo;
   int seqlen, nseq, heads;
-  float scale_log2, inv_scale_log2;
+  float scale_log2;
   int C;          // column distance between the q, k and v blocks of the packed matrix
   int qtiles;     // 128-row query tiles per sequence
-  int ngroups;    // SHARED: CTA items per (sequence, head)
-  int nitems;     // SHARED: nseq*heads*ngroups (CTA items); else nseq*heads*qtiles (slot items)
+  int nitems;     // nseq*heads*qtiles (slot items)
 };
 
-template <int DH, bool SHARED>
+template <int DH>
 struct Geo {
-  static constexpr int STAGES = SHARED ? 6 : 4;
-  static constexpr int NRINGS = SHARED ? 1 : SLOTS;
+  static constexpr int STAGES = 4;
+  static constexpr int NRINGS = SLOTS;
   static constexpr int Q_BYTES = BM * DH * 2;
   static constexpr int KV_BYTES = BK * DH * 2;                 // one K (or V) chunk
   static constexpr int STAGE_BYTES = 2 * KV_BYTES;
@@ -254,24 +145,22 @@ struct Geo {
   static constexpr uint32_t SLOT_COLS = 128;                   // S 64 | P 32 | O DH (<= 32): four slots fill the 512 columns
 };
 
-template <typename T, int DH, bool SHARED, uint32_t PMASK, bool FUSED, bool LONG>   // LONG: sequences of more than one 128-row tile
+template <typename T, int DH, bool LONG>   // LONG: sequences of more than one 128-row tile
 __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                                                                 const SlotArgs p) {
-  using G = Geo<DH, SHARED>;
+  using G = Geo<DH>;
   constexpr int STAGES = G::STAGES;
   constexpr uint32_t PITCH = DH * 2;
   constexpr uint32_t LAYOUT = DH == 64 ? 2u : (DH == 32 ? 4u : 6u);   // SWIZZLE_128B / 64B / 32B
   constexpr uint32_t SBO = 8 * PITCH;
   constexpr uint32_t COL_S = 0, COL_P = 64, COL_O = 96, COL_L = 112;
-  // Head dim 16 leaves 16 TMEM columns per slot: the row sums l = sum_k P come from the tensor core too (P times a 16 x 16
-  // tile of ones, four extra N = 16 MMAs per chunk on a pipe that is ~10 % busy) instead of one FADD2 per pair in the
-  // softmax threads, whose instruction stream is what bounds the kernel; l is then the sum of the ROUNDED P, exactly what
-  // the P V product sees.  At head dim 32 the columns are taken by O and the sums stay in registers.
-  // FUSED: the ones are appended to the V tile instead - the B operand of O += P V becomes [V | 1] with N = 32 (second
-  // MN atom = the ones block, reached through the descriptor's leading byte offset), so the SAME four MMAs per chunk
-  // produce O in columns 96-111 and the row sums in columns 112-127 (a tcgen05.mma costs the same ~45 clk for any N <= 64).
+  // Head dim 16 leaves 16 TMEM columns per slot: the row sums l = sum_k P come from the tensor core too instead of one FADD2
+  // per pair in the softmax threads, whose instruction stream is what bounds the kernel.  A 16 x 16 tile of ones is appended
+  // to the V tile - the B operand of O += P V becomes [V | 1] with N = 32 (second MN atom = the ones block, reached through
+  // the descriptor's leading byte offset), so the SAME four MMAs per chunk produce O in columns 96-111 and the row sums in
+  // columns 112-127 (a tcgen05.mma costs the same ~45 clk for any N <= 64).  l is then the sum of the ROUNDED P, exactly
+  // what the P V product sees.  At head dim 32 the columns are taken by O and the sums stay in registers.
   constexpr bool SUMS = DH == 16;
-  static_assert(!FUSED || SUMS, "fused row sums need the 16 spare TMEM columns of head dim 16");
   extern __shared__ uint8_t sl_smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(sl_smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sQ = smem;                                          // [slot][2][Q_BYTES]
@@ -308,7 +197,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
     }
     for (int i = 0; i < G::NRINGS * STAGES; ++i) {
       mbar_init(&kv_full[i], 1);
-      mbar_init(&kv_empty[i], SHARED ? SLOTS : 1);
+      mbar_init(&kv_empty[i], 1);
     }
     fence_mbar_init();
   }
@@ -332,37 +221,25 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
   const uint32_t a_kv_full = a_o_free + 8 * SLOTS, a_kv_empty = a_kv_full + 8 * G::NRINGS * STAGES;
 
   const int nchunks = (p.seqlen + BK - 1) / BK;
-  const int sh_total = p.nseq * p.heads;
-  // item -> (sequence, head, query tile of slot sl); false when that slot idles during this item
-  auto decode = [&](int item, int sl, int& seq, int& head, int& qtile) -> bool {
-    if (SHARED) {
-      const int g = item / sh_total, sh = item - g * sh_total;
-      seq = sh / p.heads;
-      head = sh - seq * p.heads;
-      const int t0 = g * p.qtiles / p.ngroups, t1 = (g + 1) * p.qtiles / p.ngroups;
-      qtile = t0 + sl;
-      return qtile < t1;
-    }
-    qtile = item % p.qtiles;
-    const int sh = item / p.qtiles;
-    head = sh % p.heads;
-    seq = sh / p.heads;
-    return true;
-  };
-  // Walking items first, first + stride, ... without a division per item (independent slots: three divisions per item in
-  // every softmax thread and driver cursor were a measurable share of the 2-chunk window items): the stride is decomposed
-  // once into (sequences, heads, query tiles) and added with carries.  The lock-step mode keeps the plain decode.
   struct ItemIt {
     int seq, head, qtile;
   };
-  int st_seq = 0, st_head = 0, st_qt = 0;
-  if (!SHARED) {
-    const int per_seq = p.heads * p.qtiles, str = static_cast<int>(gridDim.x) * SLOTS;
-    st_seq = str / per_seq;
-    const int rem = str - st_seq * per_seq;
-    st_head = rem / p.qtiles;
-    st_qt = rem - st_head * p.qtiles;
-  }
+  // item -> (sequence, head, query tile)
+  auto decode = [&](int item, ItemIt& it) {
+    it.qtile = item % p.qtiles;
+    const int sh = item / p.qtiles;
+    it.head = sh % p.heads;
+    it.seq = sh / p.heads;
+  };
+  // Walking items first, first + stride, ... without a division per item (three divisions per item in every softmax thread
+  // and driver cursor were a measurable share of the 2-chunk window items): the stride is decomposed once into (sequences,
+  // heads, query tiles) and added with carries.
+  const int stride = static_cast<int>(gridDim.x) * SLOTS;
+  const int per_seq = p.heads * p.qtiles;
+  const int st_seq = stride / per_seq;
+  const int st_rem = stride - st_seq * per_seq;
+  const int st_head = st_rem / p.qtiles;
+  const int st_qt = st_rem - st_head * p.qtiles;
   auto it_advance = [&](ItemIt& it) {
     it.qtile += st_qt;
     if (it.qtile >= p.qtiles) {
@@ -376,9 +253,8 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
     }
     it.seq += st_seq;
   };
-  // CTA items (SHARED) / slot items (independent slots) of slot sl: first, first + stride, ...
-  auto first_of = [&](int sl) { return SHARED ? static_cast<int>(blockIdx.x) : static_cast<int>(blockIdx.x) * SLOTS + sl; };
-  const int stride = SHARED ? static_cast<int>(gridDim.x) : static_cast<int>(gridDim.x) * SLOTS;
+  // items of slot sl: first, first + stride, ...
+  auto first_of = [&](int sl) { return static_cast<int>(blockIdx.x) * SLOTS + sl; };
   auto count_of = [&](int sl) { const int f = first_of(sl); return f < p.nitems ? (p.nitems - f + stride - 1) / stride : 0; };
 
   if (warp >= W_DRIVER) {
@@ -390,66 +266,50 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
       // critical path of the slot - ncu of the first version (profiles/r02_attn_history.md) showed the softmax warps
       // waiting for S a quarter of their time while the lone driver thread worked through ~250 instructions per chunk at
       // one dependent instruction per 10-20 clocks - so everything per chunk is incremental: no divisions, no descriptor
-      // rebuilds, stage / phase counters that wrap by comparison.  With the shared ring the four drivers take turns at the
-      // K/V fills (fill f belongs to driver f mod 4).
+      // rebuilds, stage / phase counters that wrap by comparison.
       const int slot = warp - W_DRIVER;
       const uint32_t tslot = tmem + static_cast<uint32_t>(slot) * G::SLOT_COLS;
       constexpr bool BF = Cvt<T>::is_bf16;
       constexpr uint32_t idesc_s = umma_idesc_f16(BF, BM, BK);                 // S: N = 64 keys, Q and K both K-major
-      constexpr uint32_t idesc_o = umma_idesc_f16(BF, BM, FUSED ? 32 : DH) | (1u << 16);    // O: B (= V, or [V | ones]) is MN-major
-      constexpr uint32_t idesc_l = umma_idesc_f16(BF, BM, 16);                 // row sums: B = a 16 x 16 tile of ones
-      const int ring_id = SHARED ? 0 : slot;
-      uint8_t* ring = sRing + ring_id * STAGES * G::STAGE_BYTES;
+      constexpr uint32_t idesc_o = umma_idesc_f16(BF, BM, SUMS ? 32 : DH) | (1u << 16);    // O: B (= V, or [V | ones]) is MN-major
+      uint8_t* ring = sRing + slot * STAGES * G::STAGE_BYTES;
       const uint32_t a_ring = smem_u32(ring), a_q = smem_u32(sQ + slot * 2 * G::Q_BYTES);
-      const uint32_t rfull = a_kv_full + 8 * ring_id * STAGES, rempty = a_kv_empty + 8 * ring_id * STAGES;
+      const uint32_t rfull = a_kv_full + 8 * slot * STAGES, rempty = a_kv_empty + 8 * slot * STAGES;
       const uint32_t b_q_full = a_q_full + 16 * slot, b_q_empty = a_q_empty + 16 * slot;
       const uint32_t b_s_full = a_s_full + 8 * slot, b_s_free = a_s_free + 8 * slot, b_p_full = a_p_full + 8 * slot, b_p_empty = a_p_empty + 8 * slot;
       const uint32_t b_o_full = a_o_full + 8 * slot, b_o_free = a_o_free + 8 * slot;
       const int first = first_of(slot);
       const int n_my = count_of(slot);
       const uint32_t total = static_cast<uint32_t>(n_my) * nchunks;
-      auto active_at = [&](int i) -> bool {
-        if (!SHARED) return true;
-        if (i >= n_my) return false;
-        int seq, head, qt;
-        return decode(first + i * stride, slot, seq, head, qt);
-      };
-      // descriptors of stage 0; a stage further on adds STAGE_BYTES to the start address (and, with the fused sums, takes the
+      // descriptors of stage 0; a stage further on adds STAGE_BYTES to the start address (and, with the row sums, takes the
       // same amount off the leading byte offset that reaches the fixed block of ones)
       constexpr uint64_t STAGE_D = G::STAGE_BYTES >> 4;
-      const uint64_t qd[2] = {desc(a_q, SBO, LAYOUT), desc(a_q + G::Q_BYTES, SBO, LAYOUT)};
-      const uint64_t kd0 = desc(a_ring, SBO, LAYOUT);
+      const uint64_t qd[2] = {umma_desc(a_q, SBO, LAYOUT), umma_desc(a_q + G::Q_BYTES, SBO, LAYOUT)};
+      const uint64_t kd0 = umma_desc(a_ring, SBO, LAYOUT);
       const uint32_t vaddr0 = a_ring + G::KV_BYTES;
       uint64_t vd0[BK / 16];
 #pragma unroll
       for (int kk = 0; kk < BK / 16; ++kk) {
         const uint32_t va = vaddr0 + 16 * PITCH * kk;
-        vd0[kk] = FUSED ? desc_lbo(va, SBO, LAYOUT, smem_u32(sOnes) - va) : desc(va, SBO, LAYOUT);
+        vd0[kk] = SUMS ? umma_desc_lbo(va, SBO, LAYOUT, smem_u32(sOnes) - va) : umma_desc(va, SBO, LAYOUT);
       }
-      constexpr uint64_t V_STEP = FUSED ? (STAGE_D - (STAGE_D << 16)) : STAGE_D;
-      const uint64_t odesc = desc(smem_u32(sOnes), 256, 6u);
+      constexpr uint64_t V_STEP = SUMS ? (STAGE_D - (STAGE_D << 16)) : STAGE_D;
 
-      // ---- loads.  K/V: fills f = l_f, l_f + LSTEP, ... of the ring (stage f mod STAGES, round f / STAGES)
-      constexpr int LSTEP = SHARED ? SLOTS : 1;
-      static_assert(LSTEP < STAGES, "one wrap per step");
-      uint32_t l_f = SHARED ? static_cast<uint32_t>(slot) : 0u, l_st = l_f, l_ph = 0;
-      int l_i = 0, l_j = static_cast<int>(l_f), l_row = 0, l_col = 0;
+      // ---- loads.  K/V: fill f of the ring goes to stage f mod STAGES in round f / STAGES
+      uint32_t l_f = 0, l_st = 0, l_ph = 0;
+      int l_i = 0, l_j = 0, l_row = 0, l_col = 0;
       ItemIt l_it{0, 0, 0}, q_it{0, 0, 0};
-      if (!SHARED && n_my > 0) {
-        decode(first, slot, l_it.seq, l_it.head, l_it.qtile);
+      if (n_my > 0) {
+        decode(first, l_it);
         q_it = l_it;
       }
       auto l_seek = [&]() {                                          // normalise (l_i, l_j) and look up the item's K/V rows
         while (l_j >= nchunks) {
           l_j -= nchunks;
           ++l_i;
-          if (!SHARED) it_advance(l_it);
+          it_advance(l_it);
         }
         if (l_i < n_my) {
-          if (SHARED) {
-            int qt;
-            decode(first + l_i * stride, slot, l_it.seq, l_it.head, qt);
-          }
           l_row = l_it.seq * p.seqlen;
           l_col = l_it.head * DH;
         }
@@ -463,13 +323,13 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
           expect_tx_a(rfull + 8 * l_st, G::STAGE_BYTES);
           tma_2d_a(dst, &tmKV, rfull + 8 * l_st, p.C + l_col, row);
           tma_2d_a(dst + G::KV_BYTES, &tmKV, rfull + 8 * l_st, 2 * p.C + l_col, row);
-          l_f += LSTEP;
-          l_st += LSTEP;
+          ++l_f;
+          ++l_st;
           if (l_st >= static_cast<uint32_t>(STAGES)) {
             l_st -= STAGES;
             l_ph ^= 1u;
           }
-          l_j += LSTEP;
+          ++l_j;
           if (l_j >= nchunks) l_seek();
         }
       };
@@ -477,57 +337,43 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
       uint32_t aq = 0;                 // Q tiles requested
       int q_i = 0;                     // next item whose Q tile is to be requested
       auto load_next_q = [&]() {
-        int seq = 0, head = 0, qt = 0;
-        if (SHARED) {
-          while (q_i < n_my && !decode(first + q_i * stride, slot, seq, head, qt)) ++q_i;
-        } else {
-          seq = q_it.seq; head = q_it.head; qt = q_it.qtile;
-        }
         if (q_i >= n_my) return;
         const uint32_t buf = aq & 1;
         if (aq >= 2) SL_WAIT(b_q_empty + 8 * buf, ((aq >> 1) - 1) & 1);
         expect_tx_a(b_q_full + 8 * buf, G::Q_BYTES);
-        tma_2d_a(a_q + buf * G::Q_BYTES, &tmQ, b_q_full + 8 * buf, head * DH, seq * p.seqlen + qt * BM);
+        tma_2d_a(a_q + buf * G::Q_BYTES, &tmQ, b_q_full + 8 * buf, q_it.head * DH, q_it.seq * p.seqlen + q_it.qtile * BM);
         ++aq;
         ++q_i;
-        if (!SHARED) it_advance(q_it);
+        it_advance(q_it);
       };
 
-      int sj = 0, si = 0, pj = 0, pi = 0;
-      bool s_act = active_at(0), p_act = s_act;
+      int sj = 0, pj = 0;
       uint32_t s_st = 0, s_ph = 0, p_st = 0;
-      uint32_t sc = 0, pc = 0;
-      uint32_t n_s = 0, n_pv = 0;      // S / PV issued by this slot (active items only)
-      uint32_t as_item = 0;            // active items whose S phase has started / completed
-      uint32_t n_item = 0;             // active items completed (o_full committed)
+      uint32_t sc = 0, pc = 0;         // S / PV issued by this slot
+      uint32_t as_item = 0;            // items whose S phase has completed
+      uint32_t n_item = 0;             // items completed (o_full committed)
       auto issue_s = [&]() {           // S(sc) = Q K^T
         // The fill this S needs may be one this very thread still owes (its stage was not free at the last probe): keep
         // probing the ring while waiting - a blocking wait here could wait for itself.
         while (!try_wait_a(rfull + 8 * s_st, s_ph)) top_up();
-        if (s_act) {
-          const uint32_t buf = as_item & 1;
-          if (sj == 0) SL_WAIT(b_q_full + 8 * buf, (as_item >> 1) & 1);
-          if (n_s > 0) SL_WAIT(b_s_free, (n_s - 1) & 1);             // the softmax warps pulled the previous S out of TMEM
-          tc_fence_after();
-          const uint64_t kdesc = kd0 + STAGE_D * s_st;
+        const uint32_t buf = as_item & 1;
+        if (sj == 0) SL_WAIT(b_q_full + 8 * buf, (as_item >> 1) & 1);
+        if (sc > 0) SL_WAIT(b_s_free, (sc - 1) & 1);                 // the softmax warps pulled the previous S out of TMEM
+        tc_fence_after();
+        const uint64_t kdesc = kd0 + STAGE_D * s_st;
 #pragma unroll
-          for (int kk = 0; kk < DH / 16; ++kk) umma_f16_ss(tslot + COL_S, qd[buf] + 2 * kk, kdesc + 2 * kk, idesc_s, kk != 0 ? 1u : 0u);
-          commit_a(b_s_full);
-          ++n_s;
-          if (sj + 1 == nchunks) {                                   // last S of the item: its Q buffer may be refilled once these MMAs are done
-            commit_a(b_q_empty + 8 * buf);
-            ++as_item;
-          }
+        for (int kk = 0; kk < DH / 16; ++kk) umma_f16_ss(tslot + COL_S, qd[buf] + 2 * kk, kdesc + 2 * kk, idesc_s, kk != 0 ? 1u : 0u);
+        commit_a(b_s_full);
+        if (sj + 1 == nchunks) {                                     // last S of the item: its Q buffer may be refilled once these MMAs are done
+          commit_a(b_q_empty + 8 * buf);
+          ++as_item;
         }
         ++sc;
         if (++s_st == static_cast<uint32_t>(STAGES)) {
           s_st = 0;
           s_ph ^= 1u;
         }
-        if (++sj == nchunks) {
-          sj = 0;
-          s_act = active_at(++si);
-        }
+        if (++sj == nchunks) sj = 0;
       };
       load_next_q();
       load_next_q();
@@ -536,34 +382,23 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
       while (pc < total) {
         top_up();
         if (sc < total) issue_s();                                   // S(pc + 1) runs while the softmax warps work on S(pc)
-        if (p_act) {
-          SL_WAIT(b_p_full, n_pv & 1);                               // P(pc) is in TMEM, O carries the current reference maximum
-          if (pj == 0 && n_item > 0) SL_WAIT(b_o_free, (n_item - 1) & 1);   // the previous item's O has been read out
-          tc_fence_after();
-          const uint32_t acc0 = pj != 0 ? 1u : 0u;
+        SL_WAIT(b_p_full, pc & 1);                                   // P(pc) is in TMEM, O carries the current reference maximum
+        if (pj == 0 && n_item > 0) SL_WAIT(b_o_free, (n_item - 1) & 1);   // the previous item's O has been read out
+        tc_fence_after();
+        const uint32_t acc0 = pj != 0 ? 1u : 0u;
 #pragma unroll
-          for (int kk = 0; kk < BK / 16; ++kk) {                     // 16 keys per MMA: A advances 8 TMEM columns, B 16 rows
-            const uint32_t acc = kk != 0 ? 1u : acc0;
-            mma_ts(tslot + COL_O, tslot + COL_P + 8 * kk, vd0[kk] + V_STEP * p_st, idesc_o, acc);
-            if (SUMS && !FUSED) mma_ts(tslot + COL_L, tslot + COL_P + 8 * kk, odesc, idesc_l, acc);   // row sums of the rounded P
-          }
-          commit_a(b_p_empty);
-          commit_a(rempty + 8 * p_st);
-          ++n_pv;
-          if (pj + 1 == nchunks) {
-            commit_a(b_o_full);
-            ++n_item;
-            load_next_q();                                           // the Q buffer of the item before this one is free by now
-          }
-        } else {
-          arrive_a(rempty + 8 * p_st);                               // an idle slot of a lock-step item still releases the stage
+        for (int kk = 0; kk < BK / 16; ++kk)                         // 16 keys per MMA: A advances 8 TMEM columns, B 16 rows
+          umma_f16_ts(tslot + COL_O, tslot + COL_P + 8 * kk, vd0[kk] + V_STEP * p_st, idesc_o, kk != 0 ? 1u : acc0);
+        commit_a(b_p_empty);
+        commit_a(rempty + 8 * p_st);
+        if (pj + 1 == nchunks) {
+          commit_a(b_o_full);
+          ++n_item;
+          load_next_q();                                             // the Q buffer of the item before this one is free by now
         }
         ++pc;
         if (++p_st == static_cast<uint32_t>(STAGES)) p_st = 0;
-        if (++pj == nchunks) {
-          pj = 0;
-          p_act = active_at(++pi);
-        }
+        if (++pj == nchunks) pj = 0;
       }
     }
   } else {
@@ -576,13 +411,13 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
     const int r = quarter * 32 + lane;
     const uint32_t tbase = tslot + (static_cast<uint32_t>(quarter * 32) << 16);
     const float c = p.scale_log2;
-    const uint64_t c2 = pk2(c, c);
+    const uint64_t c2 = f2_pack(c, c);
     const uint32_t b_s_full = a_s_full + 8 * slot, b_s_free = a_s_free + 8 * slot, b_p_full = a_p_full + 8 * slot, b_p_empty = a_p_empty + 8 * slot;
     const uint32_t b_o_full = a_o_full + 8 * slot, b_o_free = a_o_free + 8 * slot;
     const bool elected = lane == 0;
     uint32_t n_c = 0, n_item = 0;
     ItemIt s_it{0, 0, 0};
-    if (!SHARED && first < p.nitems) decode(first, slot, s_it.seq, s_it.head, s_it.qtile);
+    if (first < p.nitems) decode(first, s_it);
     // The epilogue of an item (wait for its last P V, read O and the row sum, store) is DEFERRED into the first chunk of the
     // slot's next item, between that chunk's exponentials and its P store: the P V round trip (driver wake-up + 4 MMAs +
     // commit, ~600 clk; 10 % of all samples of the 2-chunk window items sat in that wait) then hides behind exponentials.
@@ -603,7 +438,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
         inv = 1.f / l8[0];
       } else {
         float l0, l1;
-        upk2(pend_lsum2, l0, l1);
+        f2_unpack(pend_lsum2, l0, l1);
         inv = 1.f / (l0 + l1);
       }
       U8 ov[DH / 16];
@@ -627,13 +462,8 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
       pend = false;
     };
     for (int item = first; item < p.nitems; item += stride) {
-      int seq, head, qtile;
-      if (SHARED) {
-        if (!decode(item, slot, seq, head, qtile)) continue;
-      } else {
-        seq = s_it.seq; head = s_it.head; qtile = s_it.qtile;
-        it_advance(s_it);
-      }
+      const int seq = s_it.seq, head = s_it.head, qtile = s_it.qtile;
+      it_advance(s_it);
       // A warp whose 32 rows all lie beyond the sequence (the second half of the last 128-row tile of a 1600-token sequence:
       // 2 of 52 warp-tiles) only keeps the barrier protocol going: no TMEM traffic, no exponentials, nothing stored.
       if (LONG && qtile * BM + quarter * 32 >= p.seqlen) {
@@ -650,13 +480,13 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
         continue;
       }
       float m_ref = -INFINITY;
-      uint64_t lsum2 = pk2(0.f, 0.f);
+      uint64_t lsum2 = f2_pack(0.f, 0.f);
       for (int j = 0; j < nchunks; ++j, ++n_c) {
         float v[64];
         SL_WAIT(b_s_full, n_c & 1);
         tc_fence_after();
-        ld_x32(tbase + COL_S, v);
-        ld_x32(tbase + COL_S + 32, v + 32);
+        tmem_ld_x32(tbase + COL_S, v);
+        tmem_ld_x32(tbase + COL_S + 32, v + 32);
         tmem_ld_wait();
         tc_fence_before();
         __syncwarp();
@@ -691,30 +521,23 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
         const float alpha = move ? ex2((m_ref - mchunk) * c) : 1.f;
         if (move) m_ref = mchunk;
         const float msc = m_ref * c;
-        if (!SUMS && move) lsum2 = fma2(lsum2, pk2(alpha, alpha), pk2(0.f, 0.f));
-        const uint64_t nm2 = pk2(-msc, -msc), mg2 = pk2(MAGIC - msc, MAGIC - msc);
-        const float smin = m_ref - 125.f * p.inv_scale_log2;       // raw-score floor of the polynomial path
+        if (!SUMS && move) lsum2 = f2_fma(lsum2, f2_pack(alpha, alpha), f2_pack(0.f, 0.f));
+        const uint64_t nm2 = f2_pack(-msc, -msc);
         uint32_t pk[32];
         auto group = [&](int g, auto masked_tag) {                 // keys 8g .. 8g+7 -> pk[4g .. 4g+3]
           constexpr bool MASKED = decltype(masked_tag)::value;
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
             const int i = g * 4 + q;                               // pair index: keys 2i, 2i+1
-            float e0, e1;
-            if ((PMASK >> (i & 7)) & 1u) {
-              exp2_poly_pair(v[2 * i], v[2 * i + 1], smin, c2, mg2, nm2, e0, e1);
-            } else {
-              float a0, a1;
-              upk2(fma2(pk2(v[2 * i], v[2 * i + 1]), c2, nm2), a0, a1);
-              e0 = ex2(a0);
-              e1 = ex2(a1);
-            }
+            float a0, a1;
+            f2_unpack(f2_fma(f2_pack(v[2 * i], v[2 * i + 1]), c2, nm2), a0, a1);
+            float e0 = ex2(a0), e1 = ex2(a1);
             if (MASKED) {
               e0 = 2 * i < nvalid ? e0 : 0.f;
               e1 = 2 * i + 1 < nvalid ? e1 : 0.f;
             }
             pk[i] = Cvt<T>::pack(e0, e1);
-            if (!SUMS) lsum2 = add2(lsum2, pk2(e0, e1));
+            if (!SUMS) lsum2 = f2_add(lsum2, f2_pack(e0, e1));
           }
         };
         if (nvalid == BK) {
@@ -747,12 +570,12 @@ __global__ void __launch_bounds__(THREADS, 1) attn_slots_kernel(const __grid_con
             tmem_ld_wait();
 #pragma unroll
             for (int i = 0; i < 16; ++i) u16[i] = __float_as_uint(o16[i] * alpha);
-            st_x16(tbase + COL_O + cc * 16, u16);
+            tmem_st_x16(tbase + COL_O + cc * 16, u16);
           }
         }
-        st_x16(tbase + COL_P, pk);
-        st_x16(tbase + COL_P + 16, pk + 16);
-        st_wait();
+        tmem_st_x16(tbase + COL_P, pk);
+        tmem_st_x16(tbase + COL_P + 16, pk + 16);
+        tmem_st_wait();
         tc_fence_before();
         __syncwarp();
         if (elected) arrive_a(b_p_full);
@@ -791,9 +614,9 @@ static WaitDbg* debug_buffer() {
   return dev;
 }
 
-template <typename T, int DH, bool SHARED, uint32_t PMASK, bool FUSED, bool LONG>
+template <typename T, int DH, bool LONG>
 static int launch_m(const AttnArgs& a, int C, cudaStream_t st) {
-  using G = Geo<DH, SHARED>;
+  using G = Geo<DH>;
   CUtensorMap tq, tkv;
   std::string err;
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(a.ldq), static_cast<cuuint64_t>(a.nseq) * a.seqlen};
@@ -804,70 +627,24 @@ static int launch_m(const AttnArgs& a, int C, cudaStream_t st) {
   if (tma_encode(&tkv, dt, 2, a.q, dims, strides, boxkv, DH * 2, &err)) return -3;
   SlotArgs p;
   p.dbg = debug_buffer();
-  p.o = a.o; p.ldo = a.ldo; p.seqlen = a.seqlen; p.nseq = a.nseq; p.heads = a.heads; p.scale_log2 = a.scale_log2; p.inv_scale_log2 = 1.f / a.scale_log2; p.C = C;
+  p.o = a.o; p.ldo = a.ldo; p.seqlen = a.seqlen; p.nseq = a.nseq; p.heads = a.heads; p.scale_log2 = a.scale_log2; p.C = C;
   p.qtiles = (a.seqlen + BM - 1) / BM;
-  p.ngroups = (p.qtiles + SLOTS - 1) / SLOTS;
-  const long long sh = static_cast<long long>(a.nseq) * a.heads;
-  const long long nitems = SHARED ? sh * p.ngroups : sh * p.qtiles;
+  const long long nitems = static_cast<long long>(a.nseq) * a.heads * p.qtiles;
   if (nitems > 0x7fffffffLL / 2) return -2;
   p.nitems = static_cast<int>(nitems);
   // One CTA per SM (it allocates all 512 TMEM columns): more than half of the shared memory is requested so that a second
   // CTA can never become resident and spin inside tcgen05.alloc.
   const size_t smem = std::max<size_t>(G::SMEM, 116 * 1024);
-  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_slots_kernel<T, DH, SHARED, PMASK, FUSED, LONG>), 227 * 1024)) return e;
-  const long long ctas = SHARED ? nitems : (nitems + SLOTS - 1) / SLOTS;
+  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_slots_kernel<T, DH, LONG>), 227 * 1024)) return e;
+  const long long ctas = (nitems + SLOTS - 1) / SLOTS;
   const unsigned grid = static_cast<unsigned>(std::min<long long>(ctas, current_device_sms()));
-  launch_k(attn_slots_kernel<T, DH, SHARED, PMASK, FUSED, LONG>, dim3(grid), dim3(THREADS), smem, st, tq, tkv, p);
+  launch_k(attn_slots_kernel<T, DH, LONG>, dim3(grid), dim3(THREADS), smem, st, tq, tkv, p);
   return static_cast<int>(cudaGetLastError());
-}
-
-// Which pairs (index mod 8) take the polynomial exp2.  The register-only microbenchmark is fastest at 3 of 8; the kernel, whose
-// softmax threads also pull S, store P and synchronise, is issue-bound earlier: measured 309 / 311 / 326 / 336 us with
-// 0 / 1 / 2 / 3 of 8 pairs on the polynomial (small / B = 32 global attention), 111 / 113 / 113 / 125 us for the medium
-// windows - so the default is 0 (all exponentials on the MUFU); LWDETR_B200_SLOTS_POLY = 0..3 selects for A/B runs.
-static int slots_poly() {
-  static int v = [] {
-    const char* e = getenv("LWDETR_B200_SLOTS_POLY");
-    return e ? atoi(e) : 0;
-  }();
-  return v;
-}
-
-// LWDETR_B200_SLOTS_MODE (A/B measurements): bit 0 = independent slots (own K/V ring each) for long sequences too,
-// bit 1 = fused row sums (head dim 16).  Default 3, measured on small / B = 32 global attention (profiles/r02_attn_history.md): lock-step +
-// separate sums 391 us, independent 360, lock-step + fused 358, independent + fused 336 (all with 3/8 polynomial exps).
-static int slots_mode() {
-  static int v = [] {
-    const char* e = getenv("LWDETR_B200_SLOTS_MODE");
-    return e ? atoi(e) : 3;
-  }();
-  return v;
-}
-
-template <typename T, int DH, uint32_t PMASK>
-static int launch_p(const AttnArgs& a, int C, cudaStream_t st) {
-  const int mode = slots_mode();
-  if (a.seqlen <= BM) {                              // one tile per sequence (the 100-token windows): independent slots
-    if constexpr (DH == 16) {
-      if (mode & 2) return launch_m<T, DH, false, PMASK, true, false>(a, C, st);
-    }
-    return launch_m<T, DH, false, PMASK, false, false>(a, C, st);
-  }
-  const bool indep = (mode & 1) != 0;
-  if constexpr (DH == 16) {
-    if (mode & 2) return indep ? launch_m<T, DH, false, PMASK, true, true>(a, C, st) : launch_m<T, DH, true, PMASK, true, true>(a, C, st);
-  }
-  return indep ? launch_m<T, DH, false, PMASK, false, true>(a, C, st) : launch_m<T, DH, true, PMASK, false, true>(a, C, st);
 }
 
 template <typename T, int DH>
 static int launch(const AttnArgs& a, int C, cudaStream_t st) {
-  switch (slots_poly()) {
-    case 0: return launch_p<T, DH, 0x00u>(a, C, st);
-    case 1: return launch_p<T, DH, 0x01u>(a, C, st);
-    case 2: return launch_p<T, DH, 0x11u>(a, C, st);
-    default: return launch_p<T, DH, 0x49u>(a, C, st);
-  }
+  return a.seqlen > BM ? launch_m<T, DH, true>(a, C, st) : launch_m<T, DH, false>(a, C, st);
 }
 
 }  // namespace sl

@@ -1,4 +1,5 @@
-// tcgen05 / TMA attention for long sequences (the ViT global-attention blocks, vit.py:201-204 + 130-137).
+// tcgen05 / TMA attention for long sequences at head dim 64 (the ViT global-attention blocks, vit.py:201-204 + 130-137;
+// head dims 16 and 32 take the slot kernel in attn_slots.cu).
 //
 // One CTA (one per SM, all 512 TMEM columns) owns TWO 128-row query tiles of one (sequence, head).  Q, K and V
 // tiles are fetched by TMA straight out of the packed [rows, 3C] qkv matrix (box = 128 rows x dh columns at
@@ -36,95 +37,18 @@ namespace lwb {
 
 static constexpr int TC_BM = 128;     // query rows per CTA
 static constexpr int TC_BKV = 128;    // keys per chunk
-
-__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint32_t sbo_bytes, uint32_t layout_type) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>((sbo_bytes >> 4) & 0x3FFFu) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(layout_type) << 61;
-  return d;
-}
-// D[tmem] (+)= A[tmem] * B[smem desc]
-__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld_x32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,"
-      "%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-        "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-        "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_st_x16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
-      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float ex2f(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-
 static constexpr int TC_QT = 2;                              // query tiles per CTA
 static constexpr int TC_SOFT_WARPS = 8;                      // softmax warps per tile (two threads per row)
 static constexpr int TC_THREADS2 = 32 * (3 + TC_QT * TC_SOFT_WARPS);   // TMA warp, 2 MMA warps, 16 softmax warps
 static constexpr int TC_MMA1_WARP = 2 + TC_QT * TC_SOFT_WARPS;         // issuer warp of tile 1
 static constexpr int TC_KS = 4, TC_VS = 3;                   // K / V ring depths
 
-__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr)
-               : "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
-
-// 2^x for x <= 0 on the FMA / ALU pipes (no MUFU): round-to-nearest split x = n + f, f in [-0.5, 0.5], degree-3
-// minimax polynomial for 2^f (max relative error 7.5e-5, an order of magnitude below the 16-bit rounding of P),
-// exponent patched in with an integer shift-add.  Elements whose index bit is set in POLY_MASK take this path
-// (FlashAttention-4's trick to relieve the 16 exp/clk/SM MUFU); the default mask is 0 - see DESIGN.md.
-__device__ __forceinline__ float exp2_poly(float x) {
-  x = fmaxf(x, -125.f);
-  const float xf = x + 12582912.f;                 // 1.5 * 2^23: the integer part lands in the low mantissa bits
-  const float f = x - (xf - 12582912.f);
-  float pl = fmaf(f, 0.05517164617776871f, 0.2426111251115799f);
-  pl = fmaf(pl, f, 0.6932609677314758f);
-  pl = fmaf(pl, f, 0.9999280571937561f);
-  return __int_as_float(__float_as_int(pl) + (__float_as_int(xf) << 23));
-}
-
-__device__ __forceinline__ void tmem_st_x8(uint32_t taddr, const uint32_t (&r)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-               : "memory");
-}
-
 static constexpr float TC_LAZY_LOG2 = 8.f;   // the row reference maximum moves only when exceeded by more than 2^8
 
-template <typename T, int DH, uint32_t POLY_MASK>
+template <typename T, int DH>
 __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_constant__ CUtensorMap tm, const AttnArgs p, int C) {
   constexpr int TILE_BYTES = 128 * DH * 2;                     // one 128-row tile of Q, K or V
   constexpr uint32_t PITCH = DH * 2;                           // bytes per row = swizzle span
@@ -255,6 +179,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
   } else if (tile < ntiles) {
     // -------------------------------------------------------------------- softmax / epilogue: two threads per query row
     constexpr int OC = DH / 2;                                     // O columns owned by this thread (rescale, final store)
+    static_assert(OC % 16 == 0, "the final store writes 16-column pieces");
     const int quarter = warp & 3;                                  // TMEM lane quarter this warp may access
     const int half = ((warp - 2) >> 2) & 1;                        // which 64 keys of every chunk this thread owns
     const int r = quarter * 32 + lane;
@@ -268,8 +193,8 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
       mbar_wait(&s_full[tile], j & 1);
       tc_fence_after();
       __syncwarp();
-      tmem_ld_x32(tbase + colS + half * 64, *reinterpret_cast<float(*)[32]>(&v[0]));
-      tmem_ld_x32(tbase + colS + half * 64 + 32, *reinterpret_cast<float(*)[32]>(&v[32]));
+      tmem_ld_x32(tbase + colS + half * 64, v);
+      tmem_ld_x32(tbase + colS + half * 64 + 32, v + 32);
       tmem_ld_wait();
       tc_fence_before();
       __syncwarp();                                                // 32 lanes arriving on one mbarrier word serialise:
@@ -297,7 +222,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
       const float mchunk = fmaxf(mloc, xb[xpeer]);
       // ---- lazy reference maximum: both threads of a row take the same decision from the same numbers
       const bool move = (mchunk - m_ref) * p.scale_log2 > TC_LAZY_LOG2;   // true at j = 0 (m_ref = -inf)
-      const float alpha = move ? ex2f((m_ref - mchunk) * p.scale_log2) : 1.f;
+      const float alpha = move ? ex2((m_ref - mchunk) * p.scale_log2) : 1.f;
       if (move) m_ref = mchunk;
       const float msc = m_ref * p.scale_log2;
 #pragma unroll
@@ -313,7 +238,7 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
 #pragma unroll
           for (int i = 0; i < 32; ++i) {
             const float a = fmaf(v[piece * 32 + i], p.scale_log2, -msc);
-            const float x = ((POLY_MASK >> (i & 15)) & 1u) ? exp2_poly(a) : ex2f(a);
+            const float x = ex2(a);
             e[i] = (!TAIL || piece * 32 + i < kvalid) ? x : 0.f;
           }
 #pragma unroll
@@ -344,8 +269,8 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
         }
       }
       __syncwarp();
-      tmem_st_x16(tbase + colP + half * 32, *reinterpret_cast<const uint32_t(*)[16]>(&pk[0]));
-      tmem_st_x16(tbase + colP + half * 32 + 16, *reinterpret_cast<const uint32_t(*)[16]>(&pk[16]));
+      tmem_st_x16(tbase + colP + half * 32, pk);
+      tmem_st_x16(tbase + colP + half * 32 + 16, pk + 16);
       tmem_st_wait();
       tc_fence_before();
       __syncwarp();
@@ -362,31 +287,17 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
     const int qrow = q0 + tile * TC_BM + r;
     T* dst = reinterpret_cast<T*>(p.o) + (static_cast<long long>(row0) + qrow) * p.ldo + head * DH + half * OC;
     __syncwarp();
-    if constexpr (OC == 8) {
-      float o8[8];
-      tmem_ld_x8(tbase + colO + half * OC, o8);
+#pragma unroll
+    for (int c = 0; c < OC / 16; ++c) {
+      float o16[16];
+      __syncwarp();
+      tmem_ld_x16(tbase + colO + half * OC + c * 16, o16);
       tmem_ld_wait();
       if (qrow < p.seqlen) {
-        U4 o;
-        o.x = Cvt<T>::pack(o8[0] * inv, o8[1] * inv);
-        o.y = Cvt<T>::pack(o8[2] * inv, o8[3] * inv);
-        o.z = Cvt<T>::pack(o8[4] * inv, o8[5] * inv);
-        o.w = Cvt<T>::pack(o8[6] * inv, o8[7] * inv);
-        *reinterpret_cast<U4*>(dst) = o;
-      }
-    } else {
+        U8 o;
 #pragma unroll
-      for (int c = 0; c < OC / 16; ++c) {
-        float o16[16];
-        __syncwarp();
-        tmem_ld_x16(tbase + colO + half * OC + c * 16, o16);
-        tmem_ld_wait();
-        if (qrow < p.seqlen) {
-          U8 o;
-#pragma unroll
-          for (int i = 0; i < 8; ++i) o.v[i] = Cvt<T>::pack(o16[2 * i] * inv, o16[2 * i + 1] * inv);
-          stg256(dst + c * 16, o);
-        }
+        for (int i = 0; i < 8; ++i) o.v[i] = Cvt<T>::pack(o16[2 * i] * inv, o16[2 * i + 1] * inv);
+        stg256(dst + c * 16, o);
       }
     }
     tc_fence_before();
@@ -398,8 +309,8 @@ __global__ void __launch_bounds__(TC_THREADS2, 1) attn_tc_kernel(const __grid_co
   }
 }
 
-template <typename T, int DH, uint32_t POLY_MASK>
-static int launch_tc_m(const AttnArgs& a, int C, cudaStream_t st) {
+template <typename T, int DH>
+static int launch_tc(const AttnArgs& a, int C, cudaStream_t st) {
   CUtensorMap tm;
   std::string err;
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(a.ldq), static_cast<cuuint64_t>(a.nseq) * a.seqlen};
@@ -410,36 +321,16 @@ static int launch_tc_m(const AttnArgs& a, int C, cudaStream_t st) {
   // second CTA can never become resident and spin inside tcgen05.alloc.
   const size_t need = 1024 + static_cast<size_t>(TC_QT + TC_KS + TC_VS) * 128 * DH * 2 + 512 + 2 * 2 * 2 * 128 * sizeof(float);
   const size_t smem = std::max<size_t>(need, 116 * 1024);
-  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_tc_kernel<T, DH, POLY_MASK>), 200 * 1024)) return e;
+  if (int e = ensure_max_dyn_smem(reinterpret_cast<const void*>(attn_tc_kernel<T, DH>), 200 * 1024)) return e;
   dim3 grid((a.seqlen + TC_QT * TC_BM - 1) / (TC_QT * TC_BM), a.heads, a.nseq);
-  launch_k(attn_tc_kernel<T, DH, POLY_MASK>, dim3(grid), dim3(TC_THREADS2), smem, st, tm, a, C);
+  launch_k(attn_tc_kernel<T, DH>, dim3(grid), dim3(TC_THREADS2), smem, st, tm, a, C);
   return static_cast<int>(cudaGetLastError());
 }
 
-// Which score elements (index mod 16) take the polynomial exp2 instead of the MUFU.  Measured on B200 (r01e):
-// 0x8888 (25 %) gains 3 % at dh = 64 and loses 8 % at dh <= 32, where the issue slots - not the MUFU - are the
-// scarcer resource of the softmax warps; the default is therefore 0.
-#ifndef LWB_ATTN_POLY_MASK
-#define LWB_ATTN_POLY_MASK 0u
-#endif
-
-template <typename T, int DH>
-static int launch_tc(const AttnArgs& a, int C, cudaStream_t st) {
-  return launch_tc_m<T, DH, LWB_ATTN_POLY_MASK>(a, C, st);
-}
-
-// Packed-qkv fast path: q, k, v are the column blocks [0,C), [C,2C), [2C,3C) of one 16-bit matrix.
+// Packed-qkv path at head dim 64: q, k, v are the column blocks [0,C), [C,2C), [2C,3C) of one 16-bit matrix.
 int attention_tc_launch(int dtype, const AttnArgs& a, int dh, int C, cudaStream_t st) {
-  if (dtype == DT_BF16) {
-    if (dh == 16) return launch_tc<__nv_bfloat16, 16>(a, C, st);
-    if (dh == 32) return launch_tc<__nv_bfloat16, 32>(a, C, st);
-    if (dh == 64) return launch_tc<__nv_bfloat16, 64>(a, C, st);
-  } else {
-    if (dh == 16) return launch_tc<__half, 16>(a, C, st);
-    if (dh == 32) return launch_tc<__half, 32>(a, C, st);
-    if (dh == 64) return launch_tc<__half, 64>(a, C, st);
-  }
-  return -2;
+  if (dh != 64) return -2;
+  return dtype == DT_BF16 ? launch_tc<__nv_bfloat16, 64>(a, C, st) : launch_tc<__half, 64>(a, C, st);
 }
 
 }  // namespace lwb

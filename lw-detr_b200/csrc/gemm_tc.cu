@@ -18,7 +18,6 @@
 
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 namespace lwb {
@@ -727,7 +726,6 @@ int gemm_build(const GemmDesc& d, GemmOp* op, std::string* err) {
   // epilogue groups on alternate tiles once a CTA pair has at least six tiles to walk (see the kernel); the LayerNorm
   // partials a producer writes per row follow: one per (n-tile, column half) or one per (n-tile, column half, group)
   a.epi_groups = ptiles >= 6LL * (op->grid / 2) ? 2 : 1;
-  if (const char* e = getenv("LWDETR_B200_GEMM_GROUPS")) a.epi_groups = atoi(e) == 2 ? 2 : 1;   // A/B measurements
   a.stats_parts_out = a.n_tiles * (a.epi_groups == 2 ? 2 : 4);
   op->flops = 2.0 * d.M * static_cast<double>(d.N) * d.K;
   return 0;

@@ -207,6 +207,15 @@ __device__ __forceinline__ void umma_f16_ss(uint32_t tmem_d, uint64_t adesc, uin
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem desc]: the A operand (e.g. attention's P) is read straight from TMEM.
+__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrive on an mbarrier once every previously issued tcgen05.mma of this thread has completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -224,7 +233,45 @@ __device__ __forceinline__ void tmem_ld_x16(uint32_t taddr, float (&v)[16]) {
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
 }
+// 32 lanes x 32 consecutive fp32 columns into v[0..31].
+__device__ __forceinline__ void tmem_ld_x32(uint32_t taddr, float* v) {
+  uint32_t r[32];
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,"
+      "%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
+        "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
+        "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+      : "r"(taddr)
+      : "memory");
+#pragma unroll
+  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_ld_x8(uint32_t taddr, float (&v)[8]) {
+  uint32_t r[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr)
+               : "memory");
+#pragma unroll
+  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// 32 lanes x 16 consecutive 32-bit columns from r[0..15]: thread t of the warp writes row (lane_base + t).
+__device__ __forceinline__ void tmem_st_x16(uint32_t taddr, const uint32_t* r) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]),
+      "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st_x8(uint32_t taddr, const uint32_t (&r)[8]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
+               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // Shared-memory matrix descriptor for a K-major bf16/fp16 tile stored as 128-byte rows with the
 // 128B TMA swizzle (8-row x 128 B atoms, 1024 B apart): SBO = 1024 B, LBO unused (=1), version 1.
@@ -235,6 +282,27 @@ __device__ __forceinline__ uint64_t umma_desc_k128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(1024 >> 4) << 32;    // stride byte offset between 8-row groups
   d |= static_cast<uint64_t>(1) << 46;            // descriptor version (Blackwell)
   d |= static_cast<uint64_t>(2) << 61;            // SWIZZLE_128B
+  return d;
+}
+// The same for any swizzle: SBO = byte distance between 8-row groups, layout_type = 2 / 4 / 6 for SWIZZLE_128B / 64B / 32B.
+__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint32_t sbo_bytes, uint32_t layout_type) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
+  d |= static_cast<uint64_t>(1) << 16;
+  d |= static_cast<uint64_t>((sbo_bytes >> 4) & 0x3FFFu) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(layout_type) << 61;
+  return d;
+}
+// ... with an explicit leading byte offset: for an MN-major operand that is the distance between two 16-element (32-byte)
+// atoms along N - the attention slot kernel uses it to append a constant block of ones to the V tile.
+__device__ __forceinline__ uint64_t umma_desc_lbo(uint32_t smem_addr, uint32_t sbo_bytes, uint32_t layout_type, uint32_t lbo_bytes) {
+  uint64_t d = 0;
+  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
+  d |= static_cast<uint64_t>((lbo_bytes >> 4) & 0x3FFFu) << 16;
+  d |= static_cast<uint64_t>((sbo_bytes >> 4) & 0x3FFFu) << 32;
+  d |= static_cast<uint64_t>(1) << 46;
+  d |= static_cast<uint64_t>(layout_type) << 61;
   return d;
 }
 // kind::f16 instruction descriptor: fp32 accumulate, A/B both K-major.
@@ -267,26 +335,11 @@ __device__ __forceinline__ uint64_t f2_mul(uint64_t a, uint64_t b) {
   return d;
 }
 
-// 2^(s*c - m) for a PAIR of scores without the MUFU (the exp-bound attention kernels move a fraction of their exponentials
-// to the FMA pipe): t = round(s*c - m) + 1.5*2^23 by one FFMA2, the fraction f = s*c - m - round(..) in [-0.5, 0.5] by
-// two more, a degree-3 polynomial for 2^f (max relative error 7.5e-5, an order of magnitude below the 16-bit rounding
-// of P) and the integer part added into the exponent field.  The raw scores are clamped at smin = (m - 125)/c first:
-// below that 2^x is 0 for every purpose here, and an unclamped argument would wrap the exponent field.
-__device__ __forceinline__ void exp2_poly2(float s0, float s1, float smin, uint64_t c2, uint64_t magic_minus_m2, uint64_t negm2, float& e0, float& e1) {
-  constexpr float kMagic = 12582912.f;   // 1.5 * 2^23
-  const uint64_t s2 = f2_pack(fmaxf(s0, smin), fmaxf(s1, smin));
-  const uint64_t t2 = f2_fma(s2, c2, magic_minus_m2);
-  const uint64_t r2 = f2_add(t2, f2_pack(-kMagic, -kMagic));
-  const uint64_t u2 = f2_fma(r2, f2_pack(-1.f, -1.f), negm2);
-  const uint64_t f2 = f2_fma(s2, c2, u2);
-  uint64_t p2 = f2_fma(f2, f2_pack(0.05517164617776871f, 0.05517164617776871f), f2_pack(0.2426111251115799f, 0.2426111251115799f));
-  p2 = f2_fma(p2, f2, f2_pack(0.6932609677314758f, 0.6932609677314758f));
-  p2 = f2_fma(p2, f2, f2_pack(0.9999280571937561f, 0.9999280571937561f));
-  float p0, p1, t0, t1;
-  f2_unpack(p2, p0, p1);
-  f2_unpack(t2, t0, t1);
-  e0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
-  e1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
+// 2^x on the MUFU (flushes denormals; 2^-inf = 0)
+__device__ __forceinline__ float ex2(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
 }
 
 // ----------------------------------------------------------------------------- 16/32-byte global access

@@ -27,10 +27,11 @@ REL_L2 = {torch.float16: 1e-3, torch.bfloat16: 8e-3}
 @pytest.mark.parametrize("nseq,seqlen,heads,dh", [(32, 100, 12, 16), (2, 1600, 12, 16), (16, 100, 12, 32), (1, 1600, 12, 32),
                                                   (16, 100, 12, 64), (1, 1600, 12, 64), (3, 300, 8, 32), (2, 100, 8, 32),
                                                   (2, 300, 12, 32), (5, 37, 4, 16),
-                                                  # tcgen05 path (packed qkv, seqlen >= 512, dh >= 32): ragged tails, single-tile last CTA
+                                                  # attn_tc.cu (packed qkv, seqlen >= 512, dh 64): ragged tails, single-tile last CTA;
+                                                  # dh 32 at these lengths: slot kernel, ragged tails
                                                   (2, 700, 6, 32), (3, 640, 4, 64), (2, 520, 4, 32), (1, 1153, 4, 64),
-                                                  # slot kernel (attn_slots.cu: packed qkv, dh 16 any length, dh 32 windows): lock-step groups of
-                                                  # 1-4 query tiles, ragged key tails, more (window, head) items than slots, single-item launches
+                                                  # slot kernel (attn_slots.cu: packed qkv, dh 16 / 32, any length): ragged query and key
+                                                  # tails, more (sequence, head, query tile) items than slots, single-item launches
                                                   (3, 300, 4, 16), (2, 129, 4, 16), (1, 1153, 4, 16), (2, 513, 12, 16), (1, 64, 4, 16), (7, 128, 4, 16),
                                                   (640, 100, 12, 16), (70, 100, 12, 32), (3, 1, 4, 16), (2, 65, 4, 32)])
 def test_attention_matches_softmax_reference(dt, nseq, seqlen, heads, dh):

@@ -1,7 +1,6 @@
-"""CPU re-statements (numpy, float32 arithmetic where the kernels use it) of three pieces of device arithmetic whose error
+"""CPU re-statements (numpy, float32 arithmetic where the kernels use it) of two pieces of device arithmetic whose error
 bounds DESIGN.md / the kernel comments state - so that the bounds are checked, not only claimed:
   * the exact-erf GELU polynomial of the fc1 epilogue (gemm_tc.cu: gelu_erf2),
-  * the degree-3 exp2 polynomial of the attention kernels (ptx.cuh: exp2_poly2),
   * the shifted per-slice LayerNorm statistics and their combination in the consuming GEMM (gemm_tc.cu epilogue)."""
 import math
 
@@ -31,27 +30,6 @@ def test_gelu_polynomial_matches_exact_erf_gelu():
     assert (err[big] / np.abs(ref[big])).max() < 4.9e-4
     pos = x > 0.05
     assert (err[pos] / np.abs(ref[pos])).max() < 1.0e-4
-
-
-def test_exp2_polynomial_relative_error():
-    # ptx.cuh exp2_poly2: t = round(y) via the 1.5*2^23 magic add, f = y - round(y) in [-0.5, 0.5], degree-3 polynomial for 2^f,
-    # integer part added into the exponent field
-    magic = f32(12582912.0)
-    y = np.linspace(-24.0, 0.0, 400001).astype(f32)             # the range the softmax produces (scores minus the reference maximum)
-    t = (y + magic).astype(f32)
-    r = (t - magic).astype(f32)
-    f = (y - r).astype(f32)
-    assert np.abs(f).max() <= 0.5 + 1e-6
-    p = (f * f32(0.05517164617776871) + f32(0.2426111251115799)).astype(f32)
-    p = (p * f + f32(0.6932609677314758)).astype(f32)
-    p = (p * f + f32(0.9999280571937561)).astype(f32)
-    bits = p.view(np.int32) + (t.view(np.int32) << 23)          # the low mantissa bits of t hold round(y) (two's complement wrap intended)
-    got = bits.astype(np.int32).view(np.float32).astype(np.float64)
-    ref = np.exp2(y.astype(np.float64))
-    rel = np.abs(got - ref) / ref
-    assert rel.max() < 1.0e-4                                   # stated: max relative error 7.5e-5
-    # an order of magnitude below the relative rounding error of the 16-bit P it is rounded to (fp16: 4.9e-4, bf16: 3.9e-3)
-    assert rel.max() < 4.9e-4 / 4
 
 
 def _producer_partials(row, parts):

@@ -41,12 +41,22 @@ def _sel(table, prefix):
     return {k: v for k, v in table.items() if prefix in k}
 
 
-def test_attention_slot_kernels_are_tcgen05_tma_only(table):
+def test_attention_slot_kernels_are_exactly_the_dispatched_set_and_tcgen05_tma_only(table):
     ks = _sel(table, "attn_slots_kernel<")
-    assert len(ks) >= 16
+    # {fp16, bf16} x {head dim 16, 32} x {one tile per sequence, longer sequences}: nothing else is compiled
+    assert set(ks) == {"sl::attn_slots_kernel<%s, %d, %s>" % (t, dh, lg)
+                       for t in ("__half", "__nv_bfloat16") for dh in (16, 32) for lg in ("false", "true")}, sorted(ks)
     for name, c in ks.items():
         assert c["UTCHMMA"] > 0 and c["UTMALDG"] > 0 and c["LDTM"] > 0 and c["STTM"] > 0, name
         assert c["HMMA"] == 0 and c["LDGSTS"] == 0, name
+
+
+def test_attention_tc_kernels_are_head_dim_64_tcgen05_tma_only(table):
+    ks = _sel(table, "attn_tc_kernel<")
+    assert set(ks) == {"attn_tc_kernel<__half, 64>", "attn_tc_kernel<__nv_bfloat16, 64>"}, sorted(ks)
+    for name, c in ks.items():
+        assert c["UTCHMMA"] > 0 and c["UTMALDG"] > 0 and c["LDTM"] > 0, name
+        assert c["HMMA"] == 0, name
 
 
 def test_gemm_family_is_tcgen05_tma(table):
