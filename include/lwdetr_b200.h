@@ -163,12 +163,13 @@ LWDETR_API void lwdetr_destroy(lwdetr_handle* h);
 
 /* Pack the checkpoint: `n` named fp32 HOST tensors with the reference's state_dict names
  * (SURVEY.md 8b).  Folds BatchNorm into the convolutions, merges q/v biases, concatenates the
- * deformable-attention projections, resizes the position embedding, converts to the compute dtype
- * and uploads.  Synchronous.  May be called again after the weights change. */
+ * deformable-attention projections, resizes the position embedding to cfg.img_size (the raw table is kept for
+ * lwdetr_forward_at), converts to the compute dtype and uploads.  Synchronous.  May be called again after the weights
+ * change. */
 LWDETR_API int lwdetr_load_weights(lwdetr_handle* h, int n, const char* const* names, const float* const* data,
                                    const int64_t* numel);
 
-/* images: DEVICE [B, 3, S, S], fp32 (images_fp32 = 1) or the compute dtype; outputs: DEVICE fp32
+/* images: DEVICE [B, 3, S, S] with S = cfg.img_size, fp32 (images_fp32 = 1) or the compute dtype; outputs: DEVICE fp32
  * pred_logits [B, nq, num_classes], pred_boxes [B, nq, 4]; aux may be NULL.  topk_override: DEVICE
  * int32 [B, nq] or NULL - test hook that forces the two-stage selection (SURVEY.md 8c tier T2). */
 LWDETR_API int lwdetr_forward(lwdetr_handle* h, const void* images, int images_fp32, int B, float* pred_logits,
@@ -193,10 +194,23 @@ typedef struct {
 LWDETR_API int lwdetr_forward_ex(lwdetr_handle* h, const lwdetr_input* input, int B, float* pred_logits, float* pred_boxes,
                                  const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream);
 
+/* The same forward at a chosen square input resolution: images (and padding_mask) are [B, ., img_size, img_size] with
+ * img_size a multiple of 64 in [LWDETR_MIN_IMG_SIZE, LWDETR_MAX_IMG_SIZE] - the sizes the reference trains its models
+ * at (datasets/coco.py:133, square_resize_div_64) - or the handle's cfg.img_size.  The ViT runs on an (img_size/16)^2
+ * token grid with the position embedding resized to it (vit.py:26-54, 343-365); projector levels, proposals and the
+ * deformable attention follow the feature map sizes.  One handle serves every resolution from one weight arena: a
+ * change of (B, img_size) re-plans the schedule (and drops its CUDA graphs), exactly as a change of B does.
+ * lwdetr_forward_ex(h, ...) is lwdetr_forward_at(h, ..., cfg.img_size, ...). */
+#define LWDETR_MIN_IMG_SIZE 448
+#define LWDETR_MAX_IMG_SIZE 896
+LWDETR_API int lwdetr_forward_at(lwdetr_handle* h, const lwdetr_input* input, int img_size, int B, float* pred_logits,
+                                 float* pred_boxes, const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream);
+
 /* Multi-GPU init (SURVEY.md 8e): ONE ncclBroadcast of the packed weight arena from rank `root`, stream-ordered on
  * `stream`; the only collective of the path (images shard across ranks as independent replicas, nothing on the hot path).
  * Every rank first calls lwdetr_load_weights with tensors of the right shapes (any values on the non-root ranks): that
  * fixes the arena layout, which is a function of (config, dtype) only; the call verifies that the arena sizes agree.
+ * On success the handle's schedule is re-planned at its next forward (position tables follow the received weights).
  * `nccl_comm` is an ncclComm_t of a communicator the caller created (one rank per GPU); NCCL is resolved at run time
  * from the libnccl already loaded in the process (or dlopen("libnccl.so.2")), the library does not link it. */
 LWDETR_API int lwdetr_broadcast_weights(lwdetr_handle* h, void* nccl_comm, int root, void* stream);

@@ -6,6 +6,8 @@ fallback: if the library is missing or a call fails, a RuntimeError is raised.
 import ctypes
 import os
 
+from .config import MAX_IMG_SIZE, MIN_IMG_SIZE, input_resolution
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "liblwdetr_b200.so")
 
@@ -37,6 +39,7 @@ _SIGNATURES = {
     "lwdetr_broadcast_weights": (_i, [_vp, _vp, _i, _vp]),
     "lwdetr_weight_arena_bytes": (_i64, [_vp]),
     "lwdetr_forward_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "lwdetr_forward_at": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "lwdetr_set_option": (_i, [_vp, ctypes.c_char_p, _i]),
     "lwdetr_add_capture": (_i, [_vp, ctypes.c_char_p, _vp, _i64]),
     "lwdetr_capture_result": (_i64, [_vp, _i]),
@@ -322,16 +325,21 @@ class Engine:
         check(lib().lwdetr_set_option(self._h, name.encode(), int(value)), "lwdetr_set_option")
 
     def forward(self, images, want_aux=True, topk_override=None, mask=None, mean=IMAGENET_MEAN, std=IMAGENET_STD):
-        """images: CUDA [B,3,S,S] fp32 / compute dtype, or CUDA uint8 [B,S,S,3] (HWC, normalised on the fly with mean/std);
-        mask: CUDA bool [B,S,S] (True = padded pixel) or None.  Returns the reference's output dict (fp32 CUDA tensors)."""
+        """images: CUDA [B,3,R,R] fp32 / compute dtype, or CUDA uint8 [B,R,R,3] (HWC, normalised on the fly with mean/std),
+        where R is cfg.img_size or a multiple of 64 in [448, 896] (config.input_resolution); mask: CUDA bool [B,R,R]
+        (True = padded pixel) or None.  Returns the reference's output dict (fp32 CUDA tensors)."""
         import torch
         if images.device.type != "cuda":
             raise RuntimeError("lwdetr_b200: images must be CUDA tensors")
         if images.device != self.device:
             raise RuntimeError("lwdetr_b200: images are on %s but the engine lives on %s" % (images.device, self.device))
-        S = self.cfg.img_size
+        hwc = images.dtype == torch.uint8
+        S = int(images.shape[1 if hwc else 2]) if images.dim() == 4 else self.cfg.img_size
+        if S != self.cfg.img_size and input_resolution(S, S, self.cfg.img_size) != S:
+            raise RuntimeError("lwdetr_b200: input side %d is neither the configured %d nor a multiple of 64 in [%d, %d]"
+                               % (S, self.cfg.img_size, MIN_IMG_SIZE, MAX_IMG_SIZE))
         desc = InputDesc()
-        if images.dtype == torch.uint8:
+        if hwc:
             if images.dim() != 4 or tuple(images.shape[1:]) != (S, S, 3):
                 raise RuntimeError("lwdetr_b200: uint8 images must be [B, %d, %d, 3] (HWC), got %s" % (S, S, tuple(images.shape)))
             desc.format = IN_U8_NHWC
@@ -372,8 +380,8 @@ class Engine:
         ov = None
         if topk_override is not None:
             ov = topk_override.to(device=dev, dtype=torch.int32).contiguous()
-        check(lib().lwdetr_forward_ex(self._h, ctypes.byref(desc), B, ptr(logits), ptr(boxes),
-                                      ctypes.byref(aux) if aux is not None else None, ptr(ov), stream_ptr(self.device)), "lwdetr_forward_ex")
+        check(lib().lwdetr_forward_at(self._h, ctypes.byref(desc), S, B, ptr(logits), ptr(boxes),
+                                      ctypes.byref(aux) if aux is not None else None, ptr(ov), stream_ptr(self.device)), "lwdetr_forward_at")
         self._last_inputs = (images, ov, mk)    # keep alive until the stream has consumed them
         return res
 

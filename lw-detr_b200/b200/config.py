@@ -58,6 +58,27 @@ class LWDETRConfig:
         return tuple(sorted(i if i >= 0 else i + self.vit_depth for i in self.out_feature_indexes))
 
 
+# Square input sides the reference trains every released model at (datasets/coco.py:133,
+# make_coco_transforms_square_div_64, selected by --square_resize_div_64 in every released script).
+MIN_IMG_SIZE, MAX_IMG_SIZE = 448, 896
+
+
+def input_resolution(height, width, img_size=640):
+    """The side R at which a batch whose padded extent is height x width runs.
+
+    A square extent whose side is a multiple of 64 in [MIN_IMG_SIZE, MAX_IMG_SIZE] runs natively (R = side): the reference
+    ViT takes any token grid and resizes its position embedding to it (vit.py:26-54, 343-365), and the four windows per
+    side stay whole.  Any other extent that fits into img_size x img_size is padded to it (bottom / right, with a padding
+    mask), so R = img_size; anything else raises."""
+    if height == width and height % 64 == 0 and MIN_IMG_SIZE <= height <= MAX_IMG_SIZE:
+        return int(height)
+    if height <= img_size and width <= img_size:
+        return int(img_size)
+    raise RuntimeError("lwdetr_b200: images larger than the configured %dx%d are not supported, got %dx%d (square sides that "
+                       "are multiples of 64 in [%d, %d] run at their own size)" % (img_size, img_size, height, width,
+                                                                                   MIN_IMG_SIZE, MAX_IMG_SIZE))
+
+
 _W10 = (0, 1, 3, 6, 7, 9)
 _T10 = (2, 4, 5, 9)
 CONFIGS = {

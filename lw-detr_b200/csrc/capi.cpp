@@ -140,7 +140,7 @@ int lwdetr_msda_forward(int dtype, const void* value_hm, int64_t v_image_stride,
   a.value = value_hm; a.v_b_stride = v_image_stride; a.offs_logits = offs_logits; a.ld_ol = ld_ol; a.ref = ref; a.valid_ratio = valid_ratio;
   a.out = out; a.ld_out = ld_out; a.batch = B; a.nq = Lq; a.heads = M; a.levels = L; a.points = P; a.S = S;
   for (int l = 0; l < L; ++l) { a.lvl_h[l] = spatial_shapes_host[2 * l]; a.lvl_w[l] = spatial_shapes_host[2 * l + 1]; a.lvl_start[l] = level_start_host[l]; }
-  if (lwb::msda_plan(&a)) return fail("lwdetr_msda_forward: a feature level is wider than 840 tokens, larger than 8192 tokens, or there are too many bands");
+  if (lwb::msda_plan(&a)) return fail("lwdetr_msda_forward: a feature level is wider than 840 tokens, larger than 16384 tokens, or there are too many bands");
   int e = lwb::msda_launch(dtype, a, static_cast<cudaStream_t>(stream));
   if (e == -2) return fail("lwdetr_msda_forward: unsupported (levels, points) combination");
   if (e) return cuda_fail(e, "lwdetr_msda_forward launch");
@@ -216,25 +216,36 @@ int lwdetr_forward(lwdetr_handle* h, const void* images, int images_fp32, int B,
   std::string err;
   lwb::ForwardIn in;
   in.images = images; in.kind = images_fp32 ? lwb::IN_F32_NCHW : lwb::IN_16_NCHW;
-  if (h->eng->forward(in, B, pred_logits, pred_boxes, aux, topk_override, static_cast<cudaStream_t>(stream), &err))
+  if (h->eng->forward(in, B, h->eng->config().img_size, pred_logits, pred_boxes, aux, topk_override, static_cast<cudaStream_t>(stream), &err))
     return fail(err);
+  return 0;
+}
+
+int lwdetr_forward_at(lwdetr_handle* h, const lwdetr_input* input, int img_size, int B, float* pred_logits, float* pred_boxes,
+                      const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream) {
+  if (!h || !input || !input->images) return fail("lwdetr_forward_at: null pointer");
+  if (input->format != LWDETR_IN_F32_NCHW && input->format != LWDETR_IN_16_NCHW && input->format != LWDETR_IN_U8_NHWC)
+    return fail("lwdetr_forward_at: format must be LWDETR_IN_F32_NCHW, LWDETR_IN_16_NCHW or LWDETR_IN_U8_NHWC");
+  const bool in_range = img_size >= LWDETR_MIN_IMG_SIZE && img_size <= LWDETR_MAX_IMG_SIZE && img_size % 64 == 0;
+  if (!in_range && img_size != h->eng->config().img_size)
+    return fail("lwdetr_forward_at: img_size " + std::to_string(img_size) + " is neither a multiple of 64 in [" +
+                std::to_string(LWDETR_MIN_IMG_SIZE) + ", " + std::to_string(LWDETR_MAX_IMG_SIZE) + "] nor the handle's img_size " +
+                std::to_string(h->eng->config().img_size));
+  lwb::ForwardIn in;
+  in.images = input->images; in.kind = input->format; in.mask = input->padding_mask;
+  for (int c = 0; c < 3; ++c) {
+    in.mean[c] = input->mean[c]; in.stdv[c] = input->std[c];
+    if (input->format == LWDETR_IN_U8_NHWC && !(input->std[c] > 0.f)) return fail("lwdetr_forward_at: std must be positive");
+  }
+  std::string err;
+  if (h->eng->forward(in, B, img_size, pred_logits, pred_boxes, aux, topk_override, static_cast<cudaStream_t>(stream), &err)) return fail(err);
   return 0;
 }
 
 int lwdetr_forward_ex(lwdetr_handle* h, const lwdetr_input* input, int B, float* pred_logits, float* pred_boxes,
                       const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream) {
-  if (!h || !input || !input->images) return fail("lwdetr_forward_ex: null pointer");
-  if (input->format != LWDETR_IN_F32_NCHW && input->format != LWDETR_IN_16_NCHW && input->format != LWDETR_IN_U8_NHWC)
-    return fail("lwdetr_forward_ex: format must be LWDETR_IN_F32_NCHW, LWDETR_IN_16_NCHW or LWDETR_IN_U8_NHWC");
-  lwb::ForwardIn in;
-  in.images = input->images; in.kind = input->format; in.mask = input->padding_mask;
-  for (int c = 0; c < 3; ++c) {
-    in.mean[c] = input->mean[c]; in.stdv[c] = input->std[c];
-    if (input->format == LWDETR_IN_U8_NHWC && !(input->std[c] > 0.f)) return fail("lwdetr_forward_ex: std must be positive");
-  }
-  std::string err;
-  if (h->eng->forward(in, B, pred_logits, pred_boxes, aux, topk_override, static_cast<cudaStream_t>(stream), &err)) return fail(err);
-  return 0;
+  if (!h) return fail("lwdetr_forward_ex: null pointer");
+  return lwdetr_forward_at(h, input, h->eng->config().img_size, B, pred_logits, pred_boxes, aux, topk_override, stream);
 }
 
 // One ncclBroadcast of the packed weight arena (SURVEY.md 8b / 8e).  NCCL is not linked: the symbol is taken from the
@@ -273,6 +284,7 @@ int lwdetr_broadcast_weights(lwdetr_handle* h, void* nccl_comm, int root, void* 
   if (rc == -1) return fail(std::string("lwdetr_broadcast_weights: CUDA error: ") + cudaGetErrorString(cudaGetLastError()));
   if (rc == -2) return fail("lwdetr_broadcast_weights: ncclBroadcast failed");
   if (rc == -3) return fail("lwdetr_broadcast_weights: arena size differs from the root's (" + std::to_string(mine) + " vs " + std::to_string(roots) + " bytes): config / dtype mismatch between ranks");
+  h->eng->invalidate_plan();   // a position table planned for another resolution was built from this rank's old weights
   return 0;
 }
 

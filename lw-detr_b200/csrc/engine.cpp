@@ -110,9 +110,7 @@ void* Engine::salloc(size_t bytes) {
   return p;
 }
 
-void* Engine::upload16(const std::vector<float>& v) {
-  void* d = walloc(v.size() * 2);
-  if (!d) return nullptr;
+std::vector<uint16_t> Engine::to16(const std::vector<float>& v) const {
   std::vector<uint16_t> h(v.size());
   if (dtype_ == DT_BF16) {
     for (size_t i = 0; i < v.size(); ++i) {
@@ -125,8 +123,29 @@ void* Engine::upload16(const std::vector<float>& v) {
       std::memcpy(&h[i], &b, 2);
     }
   }
+  return h;
+}
+void* Engine::upload16(const std::vector<float>& v) {
+  void* d = walloc(v.size() * 2);
+  if (!d) return nullptr;
+  const std::vector<uint16_t> h = to16(v);
   cudaMemcpy(d, h.data(), h.size() * 2, cudaMemcpyHostToDevice);
   return d;
+}
+
+int Engine::upload_pos_table(int G, void* dst) {
+  const int C = cfg_.vit_dim, T = G * G;
+  std::vector<float> raw(static_cast<size_t>(196) * C), grid(static_cast<size_t>(T) * C), wm(static_cast<size_t>(T) * C);
+  if (cudaMemcpy(raw.data(), F_.at("pos_raw"), raw.size() * 4, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+  bicubic_resize_chlast(raw.data(), 14, C, G, grid.data());
+  const int wh = G / 4, wsz = wh * wh;
+  for (int r = 0; r < T; ++r) {   // window-major row r -> spatial (y, x)   (vit.py:353-358)
+    const int win = r / wsz, t = r % wsz;
+    const int y = (win >> 2) * wh + t / wh, x = (win & 3) * wh + t % wh;
+    std::memcpy(&wm[static_cast<size_t>(r) * C], &grid[(static_cast<size_t>(y) * G + x) * C], C * sizeof(float));
+  }
+  const std::vector<uint16_t> h = to16(wm);
+  return cudaMemcpy(dst, h.data(), h.size() * 2, cudaMemcpyHostToDevice) == cudaSuccess ? 0 : -1;
 }
 float* Engine::upload32(const std::vector<float>& v) {
   void* d = walloc(v.size() * 4);
@@ -243,16 +262,13 @@ int Engine::load_weights(const std::map<std::string, HostTensor>& w, std::string
   put16("patch.w", vec(E + "patch_embed.proj.weight", 1LL * C * 768));
   put32("patch.b", vec(E + "patch_embed.proj.bias", C));
   {
+    // the raw table (cls slot dropped, vit.py:39-40) stays in the arena: plan() resizes it for other input resolutions
     auto pe = vec(E + "pos_embed", 197LL * C);
-    std::vector<float> grid(static_cast<size_t>(T) * C), wm(static_cast<size_t>(T) * C);
-    bicubic_resize_chlast(pe.data() + C, 14, C, G, grid.data());   // drop the cls slot (vit.py:39-40)
-    const int wh = G / 4, wsz = wh * wh;
-    for (int r = 0; r < T; ++r) {   // window-major row r -> spatial (y, x)   (vit.py:353-358)
-      const int win = r / wsz, t = r % wsz;
-      const int y = (win >> 2) * wh + t / wh, x = (win & 3) * wh + t % wh;
-      std::memcpy(&wm[static_cast<size_t>(r) * C], &grid[(static_cast<size_t>(y) * G + x) * C], C * sizeof(float));
-    }
-    put16("pos", wm);
+    put32("pos_raw", std::vector<float>(pe.begin() + C, pe.end()));
+    void* p = walloc(static_cast<size_t>(T) * C * 2);   // the table at cfg.img_size, built once here
+    W_["pos"] = p;
+    if (!p) oom = true;
+    else if (!oom && upload_pos_table(G, p)) { *err = "CUDA error while building the position table"; return -1; }
   }
   for (int i = 0; i < cfg_.vit_depth; ++i) {
     const std::string b = E + "blocks." + std::to_string(i) + ".", k = "blk" + std::to_string(i) + ".";
@@ -390,9 +406,9 @@ int Engine::load_weights(const std::map<std::string, HostTensor>& w, std::string
 }
 
 // ------------------------------------------------------------------------------- schedule
-int Engine::plan(int B, std::string* err) {
+int Engine::plan(int B, int R, std::string* err) {
   const int C = cfg_.vit_dim, d = cfg_.hidden_dim, nq = cfg_.num_queries, ncls = cfg_.num_classes;
-  const int G = cfg_.img_size / 16, T = G * G, ntap = cfg_.n_taps, c2 = d / 2, heads = cfg_.vit_heads;
+  const int G = R / 16, T = G * G, ntap = cfg_.n_taps, c2 = d / 2, heads = cfg_.vit_heads;
   const int M = cfg_.ca_heads, L = cfg_.n_levels, P = cfg_.dec_points, ff = cfg_.dim_feedforward, NL = cfg_.dec_layers;
   const long long BT = 1LL * B * T;
   int lvl_hw[2] = {0, 0}, lvl_start[2] = {0, 0}, S = 0;
@@ -403,6 +419,7 @@ int Engine::plan(int B, std::string* err) {
     S += lvl_hw[l] * lvl_hw[l];
   }
   const long long BS = 1LL * B * S, BQ = 1LL * B * nq;
+  planned_B_ = 0;   // until this plan is complete, forward() must not run the old (or a half-built) schedule
   const int ldc = static_cast<int>(align_up(static_cast<size_t>(ncls), 32));   // row pitch of the fp32 class-logit buffers
   ldc_ = ldc;
   if (d / M != 16) { *err = "deformable attention head dim must be 16"; return -1; }
@@ -503,7 +520,7 @@ int Engine::plan(int B, std::string* err) {
     uint8_t* invalid_b = static_cast<uint8_t*>(salloc(static_cast<size_t>(BS)));
     uint8_t* pad_b = static_cast<uint8_t*>(salloc(static_cast<size_t>(BS)));
     {
-      const int img = cfg_.img_size;
+      const int img = R;
       const int lh0 = lvl_hw[0], lh1 = lvl_hw[1], ls0 = lvl_start[0], ls1 = lvl_start[1];
       add_op("mask_setup", [this, B, img, L, S, lh0, lh1, ls0, ls1, prop_b, invalid_b, pad_b, vr_b](cudaStream_t st) {
         const int lh[2] = {lh0, lh1}, ls[2] = {ls0, ls1};
@@ -518,7 +535,7 @@ int Engine::plan(int B, std::string* err) {
     Mat qkv = buf16(BT, 3 * C), att = buf16(BT, C), hid = buf16(BT, 4 * C);
     {
       void* a0p = a0.p;
-      const int img = cfg_.img_size;
+      const int img = R;
       add_op("patch_gather", [this, a0p, B, img, dt](cudaStream_t st) {
                if (in_.kind == IN_U8_NHWC) return patch_gather_u8_launch(dt, in_.images, in_.mean, in_.stdv, a0p, B, img, st);
                return patch_gather_launch(dt, in_.images, in_.kind == IN_F32_NCHW ? 1 : 0, a0p, B, img, st);
@@ -531,7 +548,13 @@ int Engine::plan(int B, std::string* err) {
     const bool fuse = fuse_ln_ != 0;
     Mat xcur = xa;
     {
-      GemmOpt o; o.resid = Mat{pass ? w16("pos") : nullptr, C}; o.resid_mod = T;
+      // position table: the load-time one at cfg.img_size, else one built for this grid in the workspace
+      Mat pos = R == cfg_.img_size ? Mat{pass ? w16("pos") : nullptr, C} : buf16(T, C);
+      if (pass && R != cfg_.img_size) {
+        // earlier forwards may still read the workspace on the device: let them finish before the host writes into it
+        if (cudaDeviceSynchronize() != cudaSuccess || upload_pos_table(G, pos.p)) { *err = "CUDA error while building the position table"; return -1; }
+      }
+      GemmOpt o; o.resid = pos; o.resid_mod = T;
       if (fuse) o.stats_out = stats_x;
       add_gemm("patch_embed", a0, BT, 768, "patch", C, xcur.p, xcur.ld, o);
     }
@@ -729,6 +752,7 @@ int Engine::plan(int B, std::string* err) {
   drop_graphs();
   eager_runs_ = 0;
   planned_B_ = B;
+  planned_R_ = R;
   return 0;
 }
 
@@ -749,12 +773,12 @@ int Engine::do_capture(const Op& op, cudaStream_t st) {
   return 0;
 }
 
-int Engine::forward(const ForwardIn& in, int B, float* pred_logits, float* pred_boxes, const lwdetr_aux_out* aux,
+int Engine::forward(const ForwardIn& in, int B, int R, float* pred_logits, float* pred_boxes, const lwdetr_aux_out* aux,
                     const int32_t* topk_override, cudaStream_t st, std::string* err) {
   DeviceGuard guard(device_);
   if (!weights_loaded_) { *err = "lwdetr_forward: weights not loaded"; return -1; }
   if (B <= 0) { *err = "lwdetr_forward: batch must be positive"; return -1; }
-  if (B != planned_B_ && plan(B, err)) return -1;
+  if ((B != planned_B_ || R != planned_R_) && plan(B, R, err)) return -1;
   if (!in.images) { *err = "lwdetr_forward: null images"; return -1; }
   in_ = in; in_topk_override_ = topk_override;
   // The first forward of a plan always runs eagerly (it also performs the one-time cudaFuncSetAttribute calls).

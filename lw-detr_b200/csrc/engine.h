@@ -1,5 +1,5 @@
 // LW-DETR forward engine: weight packing (folding, layout changes, 16-bit conversion) and the fixed
-// kernel schedule for one batch size.  Host-only interface; see engine.cpp.
+// kernel schedule for one (batch size, input resolution).  Host-only interface; see engine.cpp.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -39,9 +39,9 @@ struct Op {
 // One forward's input: the image batch in one of three encodings plus the optional NestedTensor padding mask.
 enum : int { IN_F32_NCHW = 0, IN_16_NCHW = 1, IN_U8_NHWC = 2 };
 struct ForwardIn {
-  const void* images = nullptr;   // DEVICE [B,3,S,S] fp32 / compute dtype, or [B,S,S,3] uint8
+  const void* images = nullptr;   // DEVICE [B,3,R,R] fp32 / compute dtype, or [B,R,R,3] uint8
   int kind = IN_F32_NCHW;
-  const uint8_t* mask = nullptr;  // DEVICE bool [B,S,S] (True = padded pixel) or null
+  const uint8_t* mask = nullptr;  // DEVICE bool [B,R,R] (True = padded pixel) or null
   float mean[3] = {0.f, 0.f, 0.f}, stdv[3] = {1.f, 1.f, 1.f};   // IN_U8_NHWC: (x/255 - mean) / std
 };
 
@@ -50,8 +50,11 @@ class Engine {
   Engine(const lwdetr_config& cfg, int dtype);
   ~Engine();
   int load_weights(const std::map<std::string, HostTensor>& w, std::string* err);
-  int forward(const ForwardIn& in, int B, float* pred_logits, float* pred_boxes,
+  // R: input side in pixels (a multiple of 64; the caller checks the supported range)
+  int forward(const ForwardIn& in, int B, int R, float* pred_logits, float* pred_boxes,
               const lwdetr_aux_out* aux, const int32_t* topk_override, cudaStream_t st, std::string* err);
+  // Forget the schedule (and the position table it built): the next forward re-plans from the current arena.
+  void invalidate_plan() { drop_graphs(); planned_B_ = 0; }
   void add_capture(const char* label, float* dst, long long cap) { captures_.push_back({label, dst, cap, -1}); }
   void clear_captures() { captures_.clear(); }
   long long capture_written(int i) const { return i < (int)captures_.size() ? captures_[i].written : -1; }
@@ -69,17 +72,21 @@ class Engine {
 
  private:
   struct DevBuf { void* p = nullptr; size_t bytes = 0; };
-  int plan(int B, std::string* err);
+  int plan(int B, int R, std::string* err);
   void* walloc(size_t bytes);      // weight arena (bump)
   void* salloc(size_t bytes);      // workspace arena (bump)
+  std::vector<uint16_t> to16(const std::vector<float>& v) const;   // round to the compute dtype
   void* upload16(const std::vector<float>& v);
+  // ViT position table of a G x G token grid -> dst (DEVICE, compute dtype, [G*G, C] in the window-major row order of the
+  // patch-embedding GEMM), built from the raw 14 x 14 table kept in the weight arena ("pos_raw").  Synchronous.
+  int upload_pos_table(int G, void* dst);
   float* upload32(const std::vector<float>& v);
   int do_capture(const Op& op, cudaStream_t st);
 
   lwdetr_config cfg_;
   int dtype_;
   int device_ = 0;    // CUDA device the engine was created on; every entry point switches to it (one handle per device)
-  int planned_B_ = 0;
+  int planned_B_ = 0, planned_R_ = 0;
   bool weights_loaded_ = false;
   int use_graph_ = 0;
   int fuse_ln_ = 1;   // ViT LayerNorms folded into the consuming GEMM's epilogue (option "fuse_layernorm")

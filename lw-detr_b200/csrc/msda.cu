@@ -172,7 +172,7 @@ __global__ void __launch_bounds__(MS_THREADS, 1) msda_fwd_kernel(const __grid_co
       // ---- this thread's samples, prepared ONCE per (item, pass) - not per band: the four corner weights (softmax weight and
       // the zero weight of out-of-image corners folded in), the clamped corner tokens relative to the level, the sample's row
       float wc[SPT][4];
-      uint32_t info[SPT];     // bits 0-12: token of the (clamped) top-left corner in its level, 13: x step, 14: y step, 16-31: floor(y) + 1 (0xffff: no weight)
+      uint32_t info[SPT];     // bits 0-13: token of the (clamped) top-left corner in its level, 14: x step, 15: y step, 16-31: floor(y) + 1 (0xffff: no weight)
       if (active) {
         float lg[LP];
         float mx = -INFINITY;
@@ -212,7 +212,7 @@ __global__ void __launch_bounds__(MS_THREADS, 1) msda_fwd_kernel(const __grid_co
           const float wy0 = y0 >= 0 ? w - w * fy : 0.f, wy1 = y0 + 1 < H ? w * fy : 0.f;
           const float wx0 = x0 >= 0 ? 1.f - fx : 0.f, wx1 = x0 + 1 < W ? fx : 0.f;
           wc[k][0] = wy0 * wx0; wc[k][1] = wy0 * wx1; wc[k][2] = wy1 * wx0; wc[k][3] = wy1 * wx1;
-          info[k] = static_cast<uint32_t>(ya * W + xa) | (static_cast<uint32_t>(xb - xa) << 13) | (static_cast<uint32_t>(yb - ya) << 14) |
+          info[k] = static_cast<uint32_t>(ya * W + xa) | (static_cast<uint32_t>(xb - xa) << 14) | (static_cast<uint32_t>(yb - ya) << 15) |
                     ((w != 0.f ? static_cast<uint32_t>(y0 + 1) : 0xffffu) << 16);   // a sample without weight never matches a band
         }
       }
@@ -232,8 +232,8 @@ __global__ void __launch_bounds__(MS_THREADS, 1) msda_fwd_kernel(const __grid_co
             const int y0 = static_cast<int>(info[ks] >> 16) - 1;
             if (y0 < own0 || y0 > own1) continue;                          // the band that holds both rows of the sample takes it
             const int W = p.lvl_w[l];
-            const uint32_t a00 = stage + static_cast<uint32_t>(static_cast<int>(info[ks] & 0x1fffu) - row0 * W) * 32u;
-            const uint32_t ax = ((info[ks] >> 13) & 1u) * 32u, ay = ((info[ks] >> 14) & 1u) * static_cast<uint32_t>(W) * 32u;
+            const uint32_t a00 = stage + static_cast<uint32_t>(static_cast<int>(info[ks] & 0x3fffu) - row0 * W) * 32u;
+            const uint32_t ax = ((info[ks] >> 14) & 1u) * 32u, ay = ((info[ks] >> 15) & 1u) * static_cast<uint32_t>(W) * 32u;
             const uint32_t addr[4] = {a00, a00 + ax, a00 + ay, a00 + ay + ax};
 #pragma unroll
             for (int rowp = 0; rowp < 2; ++rowp) {                         // the two corners of one image row at a time (16 registers in flight)
@@ -287,7 +287,7 @@ int msda_plan(MsdaArgs* a) {
   a->nbands = 0;
   for (int l = 0; l < a->levels; ++l) {
     const int H = a->lvl_h[l], W = a->lvl_w[l];
-    if (H < 1 || W < 1 || 2 * W > MS_STAGE_TOKENS || H * W > 8192 || H > 0xfff0) return -2;   // token / row fields of the packed sample info
+    if (H < 1 || W < 1 || 2 * W > MS_STAGE_TOKENS || H * W > 16384 || H > 0xfff0) return -2;   // 14-bit token / 16-bit row fields of the packed sample info
     const int rows_max = MS_STAGE_TOKENS / W;                    // rows a stage holds
     if (H <= rows_max) {
       if (a->nbands >= MSDA_MAX_BANDS) return -2;

@@ -10,7 +10,7 @@ import torch
 from torch import nn
 
 from b200 import capi
-from b200.config import config_from_args
+from b200.config import config_from_args, input_resolution
 from b200.spec import param_spec
 from util.misc import NestedTensor, nested_tensor_from_tensor_list
 
@@ -96,7 +96,9 @@ class LWDETR(nn.Module):
 
     @torch.no_grad()
     def forward(self, samples, targets=None):
-        """samples: NestedTensor | list of [3,H,W] tensors | [B,3,H,W] tensor (lwdetr.py:111-127).
+        """samples: NestedTensor | list of [3,H,W] tensors | [B,3,H,W] tensor (lwdetr.py:111-127), or uint8 [B,R,R,3] frames.
+        A square batch extent R that is a multiple of 64 in [448, 896] runs at R, as the reference does; any other extent
+        up to cfg.img_size is padded to it with a padding mask (b200.config.input_resolution).
         Returns {'pred_logits' [B,nq,C], 'pred_boxes' [B,nq,4] (cxcywh, normalised), 'aux_outputs',
         'enc_outputs'} as fp32 CUDA tensors (lwdetr.py:161-174)."""
         if self.training:
@@ -107,6 +109,8 @@ class LWDETR(nn.Module):
             dev = next(self.parameters()).device
             if dev.type != "cuda":
                 raise RuntimeError("lwdetr_b200: move the model to a CUDA device (no CPU fallback)")
+            if samples.dim() == 4:
+                self._check_export_size(input_resolution(samples.shape[1], samples.shape[2], self.cfg.img_size))
             out = self.engine().forward(samples.to(dev), want_aux=True)
             return self._pack_outputs(out)
         if isinstance(samples, (list, torch.Tensor)):
@@ -115,11 +119,12 @@ class LWDETR(nn.Module):
         dev = next(self.parameters()).device
         if dev.type != "cuda":
             raise RuntimeError("lwdetr_b200: move the model to a CUDA device (no CPU fallback)")
-        S = self.cfg.img_size
-        if x.dim() != 4 or x.shape[-1] > S or x.shape[-2] > S:
-            raise RuntimeError("lwdetr_b200: images larger than the configured %dx%d are not supported, got %s" % (S, S, tuple(x.shape)))
+        if x.dim() != 4:
+            raise RuntimeError("lwdetr_b200: expected a [B, 3, H, W] batch, got %s" % (tuple(x.shape),))
+        S = input_resolution(x.shape[-2], x.shape[-1], self.cfg.img_size)
+        self._check_export_size(S)
         if x.shape[-1] != S or x.shape[-2] != S:
-            # a batch whose largest image is smaller than the model's input: pad to the configured size (bottom / right,
+            # a batch whose extent is not a native input size: pad to the configured size (bottom / right,
             # exactly what nested_tensor_from_tensor_list does between the images of a batch) and extend the mask
             xp = x.new_zeros((x.shape[0], x.shape[1], S, S))
             xp[:, :, : x.shape[-2], : x.shape[-1]] = x
@@ -131,6 +136,11 @@ class LWDETR(nn.Module):
         mask = mask.to(dev) if (mask is not None and bool(mask.any())) else None
         out = self.engine().forward(x, want_aux=True, mask=mask)
         return self._pack_outputs(out)
+
+    def _check_export_size(self, R):
+        # the reference's forward_export adds pos_embed_export, computed once for the 40x40 grid (vit.py:328-332)
+        if self._export and R != self.cfg.img_size:
+            raise RuntimeError("lwdetr_b200: export mode runs at the configured %dx%d only, got %dx%d" % (self.cfg.img_size, self.cfg.img_size, R, R))
 
     def _pack_outputs(self, out):
         if self._export:

@@ -147,9 +147,82 @@ DEMO_SMALL_FLAGS = ("--encoder vit_tiny --vit_encoder_num_layers 10 --window_blo
                     "--two_stage --bbox_reparam --lite_refpoint_refine --num_select 300").split()     # scripts/lwdetr_small_coco_eval.sh:10-24
 
 
+RES_CASES = [("tiny", 448, 2), ("small", 512, 1), ("medium", 576, 1), ("large", 768, 1), ("xlarge", 896, 1)]
+RES_PAD_EXTENT, RES_PAD_VALID = 512, [(512, 512), (448, 384)]     # tiny, weight seed 1, image seed 9
+
+
+def res_padded_inputs():
+    """A 512x512 and a 448x384 image batched the way util/misc.py:317-339 does: padded to their common 512x512 extent."""
+    x = synth_images(2, 9, RES_PAD_EXTENT).clone()
+    mask = torch.zeros(2, RES_PAD_EXTENT, RES_PAD_EXTENT, dtype=torch.bool)
+    for b, (h, w) in enumerate(RES_PAD_VALID):
+        mask[b, h:, :] = True
+        mask[b, :, w:] = True
+        x[b][:, mask[b]] = 0
+    return x, mask
+
+
+# strided samples (sample()) keep the fixture small: logits and intermediates are sampled, boxes are stored whole.  A
+# reader recovers the stride from the stored length: sample(t, len(stored)).
+RES_LOGIT_SAMPLES, RES_ENC_LOGIT_SAMPLES, RES_FEATURE_SAMPLES = 2048, 1024, 512
+
+
+def _run_with_samples(model, cfg, inp):
+    """Reference forward: whole boxes, strided samples of the class logits and of level* / dec*."""
+    rec, hooks = {}, []
+
+    def proj_hook(m, a, o):
+        for l, f in enumerate(o):
+            rec["level%d" % l] = sample(f.flatten(2).transpose(1, 2), RES_FEATURE_SAMPLES)
+
+    hooks.append(model.backbone[0].projector.register_forward_hook(proj_hook))
+    for i, lay in enumerate(model.transformer.decoder.layers):
+        hooks.append(lay.register_forward_hook(lambda m, a, o, i=i: rec.__setitem__("dec%d" % i, sample(o, RES_FEATURE_SAMPLES))))
+    with torch.no_grad():
+        out = model(inp)
+    for h in hooks:
+        h.remove()
+    rec["pred_logits"] = sample(out["pred_logits"], RES_LOGIT_SAMPLES)
+    rec["pred_boxes"] = out["pred_boxes"].numpy()
+    rec["enc_logits"] = sample(out["enc_outputs"]["pred_logits"], RES_ENC_LOGIT_SAMPLES)
+    rec["enc_boxes"] = out["enc_outputs"]["pred_boxes"].numpy()
+    return rec
+
+
+def make_resolution_golden():
+    """ref_res.npz (about 0.2 MB): the reference at square input sizes other than 640 (its ViT resizes the position
+    embedding to the token grid, vit.py:26-54, and everything downstream follows the feature map sizes).  Keys are
+    '<case>_<field>' with
+    case '<config><R>' for RES_CASES (weights seed 1, images seed 0) and 'pad512' for a padded tiny batch (weights
+    seed 1, images seed 9); '<case>_meta' = [B, weight seed, image seed, R]."""
+    rec = {}
+    for name, R, B in RES_CASES:
+        cfg = CONFIGS[name]
+        model, _, _ = ref_import.build_reference(cfg)
+        model.load_state_dict(synth_state_dict(cfg, WEIGHT_SEED), strict=True)
+        case = "%s%d" % (name, R)
+        for k, v in _run_with_samples(model, cfg, synth_images(B, IMAGE_SEED, R)).items():
+            rec[case + "_" + k] = v
+        rec[case + "_meta"] = np.array([B, WEIGHT_SEED, IMAGE_SEED, R], dtype=np.int64)
+        print("resolution", case, rec[case + "_pred_boxes"].shape, flush=True)
+    cfg = CONFIGS["tiny"]
+    model, _, _ = ref_import.build_reference(cfg)
+    model.load_state_dict(synth_state_dict(cfg, WEIGHT_SEED), strict=True)
+    x, mask = res_padded_inputs()
+    nested = sys.modules["_ref_util.misc"].NestedTensor(x, mask)
+    for k, v in _run_with_samples(model, cfg, nested).items():
+        rec["pad512_" + k] = v
+    rec["pad512_meta"] = np.array([2, WEIGHT_SEED, 9, RES_PAD_EXTENT], dtype=np.int64)
+    rec["pad512_valid"] = np.array(RES_PAD_VALID, dtype=np.int64)
+    np.savez_compressed(os.path.join(GOLD, "ref_res.npz"), **rec)
+
+
 def main():
     torch.set_num_threads(os.cpu_count())
     os.makedirs(GOLD, exist_ok=True)
+    if "--resolution-only" in sys.argv:
+        make_resolution_golden()
+        return
     if "--postprocess-only" in sys.argv:
         make_postprocess_goldens()
         return

@@ -4,6 +4,7 @@ Prints / returns per-stage errors (SURVEY.md 8c tiers T1 pre-top-k tensors, T2 f
 T3 free-running).  Runs on the GPU box:  python tools/parity_report.py small --batch 2 --dtype fp16
 """
 import argparse
+import dataclasses
 import json
 import os
 import sys
@@ -24,16 +25,19 @@ def rel_l2(a, b):
     return ((a - b).norm() / (b.norm() + 1e-12)).item()
 
 
-def ladder(name, batch, dtype, wseed=1, iseed=0, eng=None):
+def ladder(name, batch, dtype, wseed=1, iseed=0, eng=None, img_size=640):
+    """img_size: square input side; the engine keeps the configuration's own img_size and runs at img_size through
+    lwdetr_forward_at, the oracle takes the level shapes and proposals of a config with img_size replaced."""
     cfg = CONFIGS[name]
     sd = synth_state_dict(cfg, wseed)
-    x = synth_images(batch, iseed)
-    inter = {}
-    ref = orc.forward(sd, cfg, x, inter=inter)
+    x = synth_images(batch, iseed, img_size)
     own = eng is None
     if own:
         eng = capi.Engine(cfg, dtype)
         eng.load_state_dict(sd)
+    cfg = dataclasses.replace(cfg, img_size=img_size)
+    inter = {}
+    ref = orc.forward(sd, cfg, x, inter=inter)
     xg = x.cuda()
     BT, C, d, S, nq = batch * cfg.tokens, cfg.vit_dim, cfg.hidden_dim, cfg.memory_len, cfg.num_queries
     caps = {"patch_embed": BT * C}
@@ -52,7 +56,7 @@ def ladder(name, batch, dtype, wseed=1, iseed=0, eng=None):
     torch.cuda.synchronize()
     got = eng.capture_results()
     eng.clear_captures()
-    rep = {"config": name, "batch": batch, "dtype": str(dtype).replace("torch.", "")}
+    rep = {"config": name, "batch": batch, "img_size": img_size, "dtype": str(dtype).replace("torch.", "")}
     t1 = {}
     t1["patch_embed"] = rel_l2(got["patch_embed"].reshape(BT, C), inter["patch"].reshape(BT, C))
     for i in range(cfg.vit_depth):
