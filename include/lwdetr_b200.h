@@ -194,6 +194,30 @@ typedef struct {
 LWDETR_API int lwdetr_forward_ex(lwdetr_handle* h, const lwdetr_input* input, int B, float* pred_logits, float* pred_boxes,
                                  const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream);
 
+/* The same forward on uint8 RGB frames of ANY size, each resized on the device exactly as the reference's callers resize
+ * on the host: demo/demo.py:146-159 runs transforms.Resize([640, 640]) on a PIL image, and the square_resize_div_64 eval
+ * transform (datasets/transforms.py:223-232, datasets/coco.py:149-153) is the same call.  Both are Pillow's
+ * Image.resize((S, S), BILINEAR); the result here is bit-identical to it (csrc/resize.cu states the arithmetic), and
+ * the /255, Normalize(mean, std) and patch gather of LWDETR_IN_U8_NHWC follow in the same kernel.  So the predictions
+ * are bit-identical to lwdetr_forward_at on the Pillow-resized frames, and the resize costs no host time.
+ *   frames: HOST array [B] of descriptors; each frame's pixels are DEVICE HWC RGB uint8, pixel (y, x) channel c at
+ *     data + y*row_stride + x*3 + c.  Sides in [1, LWDETR_MAX_FRAME_SIDE], row_stride >= 3*width (cropped views need
+ *     no copy), no alignment requirement; one batch may mix sizes.  B <= LWDETR_MAX_FRAMES (descriptors travel as kernel
+ *     parameters).  The frames must stay valid until the stream has consumed them.
+ *   img_size follows the rule of lwdetr_forward_at.  frames and lwdetr_forward_at share one schedule (and CUDA graph)
+ *   per (B, img_size): frames of new sizes need no re-plan.  Boxes come out normalised to the frame, as the
+ *   reference's do; scale them by each frame's (height, width) (PostProcess target_sizes) for source pixels. */
+#define LWDETR_MAX_FRAMES 1024
+#define LWDETR_MAX_FRAME_SIDE 8192
+typedef struct {
+  const uint8_t* data;   /* DEVICE, HWC RGB */
+  int32_t height, width;
+  int64_t row_stride;    /* bytes */
+} lwdetr_frame;
+LWDETR_API int lwdetr_forward_frames(lwdetr_handle* h, const lwdetr_frame* frames, int B, int img_size, const float mean[3],
+                                     const float std[3], float* pred_logits, float* pred_boxes, const lwdetr_aux_out* aux,
+                                     const int32_t* topk_override, void* stream);
+
 /* The same forward at a chosen square input resolution: images (and padding_mask) are [B, ., img_size, img_size] with
  * img_size a multiple of 64 in [LWDETR_MIN_IMG_SIZE, LWDETR_MAX_IMG_SIZE] - the sizes the reference trains its models
  * at (datasets/coco.py:133, square_resize_div_64) - or the handle's cfg.img_size.  The ViT runs on an (img_size/16)^2
@@ -226,7 +250,8 @@ LWDETR_API int lwdetr_add_capture(lwdetr_handle* h, const char* label, float* ds
 LWDETR_API int64_t lwdetr_capture_result(lwdetr_handle* h, int index);
 LWDETR_API void lwdetr_clear_captures(lwdetr_handle* h);
 
-/* Schedule introspection / per-op timing of the last planned batch size. */
+/* Schedule introspection / per-op timing of the last planned batch size.  The bytes of the input-reading op
+ * "patch_gather" are those of the last forward's input (after lwdetr_forward_frames: the frames' bytes). */
 LWDETR_API int lwdetr_num_ops(lwdetr_handle* h);
 LWDETR_API const char* lwdetr_op_label(lwdetr_handle* h, int i);
 LWDETR_API int lwdetr_op_cost(lwdetr_handle* h, int i, double* flops, double* bytes);

@@ -40,6 +40,7 @@ _SIGNATURES = {
     "lwdetr_weight_arena_bytes": (_i64, [_vp]),
     "lwdetr_forward_ex": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "lwdetr_forward_at": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "lwdetr_forward_frames": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "lwdetr_set_option": (_i, [_vp, ctypes.c_char_p, _i]),
     "lwdetr_add_capture": (_i, [_vp, ctypes.c_char_p, _vp, _i64]),
     "lwdetr_capture_result": (_i64, [_vp, _i]),
@@ -251,6 +252,14 @@ IN_F32_NCHW, IN_16_NCHW, IN_U8_NHWC = 0, 1, 2
 IMAGENET_MEAN, IMAGENET_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)      # demo/demo.py:150-153, datasets/coco.py
 
 
+class FrameDesc(ctypes.Structure):
+    """lwdetr_frame: one uint8 HWC RGB frame on the device, pixel (y, x) channel c at data + y*row_stride + x*3 + c."""
+    _fields_ = [("data", _vp), ("height", ctypes.c_int32), ("width", ctypes.c_int32), ("row_stride", ctypes.c_int64)]
+
+
+MAX_FRAMES, MAX_FRAME_SIDE = 1024, 8192      # LWDETR_MAX_FRAMES, LWDETR_MAX_FRAME_SIDE
+
+
 class AuxOut(ctypes.Structure):
     _fields_ = [(n, _vp) for n in ("aux_logits", "aux_boxes", "enc_logits", "enc_boxes", "topk_index")]
 
@@ -359,8 +368,60 @@ class Engine:
             mk = mask.to(device=self.device, dtype=torch.bool).contiguous()
         desc.images = images.data_ptr()
         desc.padding_mask = mk.data_ptr() if mk is not None else None
-        B, nq, nc, nl = images.shape[0], self.cfg.num_queries, self.cfg.num_classes, self.cfg.dec_layers
-        dev = images.device
+        B = images.shape[0]
+        res, logits, boxes, aux = self._outputs(B, want_aux)
+        ov = None
+        if topk_override is not None:
+            ov = topk_override.to(device=self.device, dtype=torch.int32).contiguous()
+        check(lib().lwdetr_forward_at(self._h, ctypes.byref(desc), S, B, ptr(logits), ptr(boxes),
+                                      ctypes.byref(aux) if aux is not None else None, ptr(ov), stream_ptr(self.device)), "lwdetr_forward_at")
+        self._last_inputs = (images, ov, mk)    # keep alive until the stream has consumed them
+        return res
+
+    def forward_frames(self, frames, img_size=None, want_aux=True, mean=IMAGENET_MEAN, std=IMAGENET_STD, topk_override=None):
+        """frames: CUDA uint8 RGB frames of any size - a [B, H, W, 3] tensor or a list of [H_i, W_i, 3] tensors, channel
+        stride 1 and pixel stride 3, any row stride (cropped views are read in place).  Each frame is resized to
+        img_size x img_size (default cfg.img_size) on the device exactly as Pillow's Image.resize((R, R), BILINEAR) -
+        torchvision's Resize([R, R]) on a PIL image - then normalised with mean/std.  Returns forward()'s dict."""
+        import torch
+        R = self.cfg.img_size if img_size is None else int(img_size)
+        if isinstance(frames, torch.Tensor):
+            if frames.dim() != 4:
+                raise RuntimeError("lwdetr_b200: frames must be [B, H, W, 3] or a list of [H, W, 3], got %s" % (tuple(frames.shape),))
+            frames = list(frames.unbind(0))
+        frames = list(frames)
+        if not 1 <= len(frames) <= MAX_FRAMES:
+            raise RuntimeError("lwdetr_b200: %d frames; a call takes 1 to %d" % (len(frames), MAX_FRAMES))
+        descs = (FrameDesc * len(frames))()
+        for i, f in enumerate(frames):
+            if not isinstance(f, torch.Tensor) or f.dtype != torch.uint8:
+                raise RuntimeError("lwdetr_b200: frame %d must be a uint8 tensor, got %s" % (i, getattr(f, "dtype", type(f))))
+            if f.device != self.device:
+                raise RuntimeError("lwdetr_b200: frame %d is on %s but the engine lives on %s" % (i, f.device, self.device))
+            if f.dim() != 3 or f.shape[2] != 3:
+                raise RuntimeError("lwdetr_b200: frame %d must be HWC RGB [H, W, 3], got %s" % (i, tuple(f.shape)))
+            H, W = int(f.shape[0]), int(f.shape[1])
+            if f.stride(2) != 1 or (W > 1 and f.stride(1) != 3):
+                raise RuntimeError("lwdetr_b200: frame %d needs channel stride 1 and pixel stride 3, got strides %s" % (i, f.stride()))
+            descs[i].data, descs[i].height, descs[i].width = f.data_ptr(), H, W
+            descs[i].row_stride = f.stride(0) if H > 1 else 3 * W      # a one-row view may report any row stride
+        m, s = (ctypes.c_float * 3)(*[float(v) for v in mean]), (ctypes.c_float * 3)(*[float(v) for v in std])
+        B = len(frames)
+        res, logits, boxes, aux = self._outputs(B, want_aux)
+        ov = None
+        if topk_override is not None:
+            ov = topk_override.to(device=self.device, dtype=torch.int32).contiguous()
+        check(lib().lwdetr_forward_frames(self._h, ctypes.cast(descs, _vp), B, R, ctypes.cast(m, _vp), ctypes.cast(s, _vp),
+                                          ptr(logits), ptr(boxes), ctypes.byref(aux) if aux is not None else None, ptr(ov),
+                                          stream_ptr(self.device)), "lwdetr_forward_frames")
+        self._last_inputs = (frames, ov, None)   # keep alive until the stream has consumed them
+        return res
+
+    def _outputs(self, B, want_aux):
+        """The result dict and the fp32 CUDA buffers the forward entry points write into."""
+        import torch
+        nq, nc, nl = self.cfg.num_queries, self.cfg.num_classes, self.cfg.dec_layers
+        dev = self.device
         logits = torch.empty(B, nq, nc, device=dev, dtype=torch.float32)
         boxes = torch.empty(B, nq, 4, device=dev, dtype=torch.float32)
         aux = None
@@ -377,13 +438,7 @@ class Engine:
             res["aux_outputs"] = [{"pred_logits": al[i], "pred_boxes": ab[i]} for i in range(nl - 1)]
             res["enc_outputs"] = {"pred_logits": el, "pred_boxes": eb}
             res["topk_index"] = ti
-        ov = None
-        if topk_override is not None:
-            ov = topk_override.to(device=dev, dtype=torch.int32).contiguous()
-        check(lib().lwdetr_forward_at(self._h, ctypes.byref(desc), S, B, ptr(logits), ptr(boxes),
-                                      ctypes.byref(aux) if aux is not None else None, ptr(ov), stream_ptr(self.device)), "lwdetr_forward_at")
-        self._last_inputs = (images, ov, mk)    # keep alive until the stream has consumed them
-        return res
+        return res, logits, boxes, aux
 
     # ---- debug captures -------------------------------------------------------------------------
     def capture(self, label, numel):

@@ -242,6 +242,37 @@ int lwdetr_forward_at(lwdetr_handle* h, const lwdetr_input* input, int img_size,
   return 0;
 }
 
+int lwdetr_forward_frames(lwdetr_handle* h, const lwdetr_frame* frames, int B, int img_size, const float mean[3], const float std[3],
+                          float* pred_logits, float* pred_boxes, const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream) {
+  if (!h || !frames || !mean || !std) return fail("lwdetr_forward_frames: null pointer");
+  if (B < 1 || B > LWDETR_MAX_FRAMES)
+    return fail("lwdetr_forward_frames: B = " + std::to_string(B) + " is outside [1, " + std::to_string(LWDETR_MAX_FRAMES) + "]");
+  const bool in_range = img_size >= LWDETR_MIN_IMG_SIZE && img_size <= LWDETR_MAX_IMG_SIZE && img_size % 64 == 0;
+  if (!in_range && img_size != h->eng->config().img_size)
+    return fail("lwdetr_forward_frames: img_size " + std::to_string(img_size) + " is neither a multiple of 64 in [" +
+                std::to_string(LWDETR_MIN_IMG_SIZE) + ", " + std::to_string(LWDETR_MAX_IMG_SIZE) + "] nor the handle's img_size " +
+                std::to_string(h->eng->config().img_size));
+  for (int i = 0; i < B; ++i) {
+    const lwdetr_frame& f = frames[i];
+    const std::string which = "lwdetr_forward_frames: frame " + std::to_string(i);
+    if (!f.data) return fail(which + " has a null data pointer");
+    if (f.height < 1 || f.width < 1 || f.height > LWDETR_MAX_FRAME_SIDE || f.width > LWDETR_MAX_FRAME_SIDE)
+      return fail(which + " is " + std::to_string(f.height) + " x " + std::to_string(f.width) + "; sides must be in [1, " +
+                  std::to_string(LWDETR_MAX_FRAME_SIDE) + "]");
+    if (f.row_stride < 3LL * f.width)
+      return fail(which + ": row_stride " + std::to_string(f.row_stride) + " is less than 3 * width = " + std::to_string(3LL * f.width));
+  }
+  lwb::ForwardIn in;
+  in.kind = lwb::IN_U8_FRAMES; in.frames = frames;
+  for (int c = 0; c < 3; ++c) {
+    in.mean[c] = mean[c]; in.stdv[c] = std[c];
+    if (!(std[c] > 0.f)) return fail("lwdetr_forward_frames: std must be positive");
+  }
+  std::string err;
+  if (h->eng->forward(in, B, img_size, pred_logits, pred_boxes, aux, topk_override, static_cast<cudaStream_t>(stream), &err)) return fail(err);
+  return 0;
+}
+
 int lwdetr_forward_ex(lwdetr_handle* h, const lwdetr_input* input, int B, float* pred_logits, float* pred_boxes,
                       const lwdetr_aux_out* aux, const int32_t* topk_override, void* stream) {
   if (!h) return fail("lwdetr_forward_ex: null pointer");

@@ -18,6 +18,7 @@
 #include "attn.h"
 #include "gemm_tc.h"
 #include "msda.h"
+#include "resize.h"
 #include "rowops.h"
 
 namespace lwb {
@@ -537,11 +538,16 @@ int Engine::plan(int B, int R, std::string* err) {
       void* a0p = a0.p;
       const int img = R;
       add_op("patch_gather", [this, a0p, B, img, dt](cudaStream_t st) {
+               if (in_.kind == IN_U8_FRAMES) return resize_patch_gather_u8_launch(dt, frames_.data(), B, img, in_.mean, in_.stdv, a0p, st);
                if (in_.kind == IN_U8_NHWC) return patch_gather_u8_launch(dt, in_.images, in_.mean, in_.stdv, a0p, B, img, st);
                return patch_gather_launch(dt, in_.images, in_.kind == IN_F32_NCHW ? 1 : 0, a0p, B, img, st);
              },
              a0.p, BT, 768, 768, 0, 1.0 * B * 3 * img * img * 4 + 2.0 * BT * 768);
-      if (pass) ops_.back().reads_input = true;
+      if (pass) {
+        ops_.back().reads_input = true;
+        patch_op_ = static_cast<int>(ops_.size()) - 1;
+        patch_bytes_ = ops_.back().bytes;
+      }
     }
     float2* stats_x = static_cast<float2*>(salloc(static_cast<size_t>(BT) * 48 * sizeof(float2)));   // row stats of x (block input)
     float2* stats_m = static_cast<float2*>(salloc(static_cast<size_t>(BT) * 48 * sizeof(float2)));   // row stats of x + attn
@@ -779,8 +785,17 @@ int Engine::forward(const ForwardIn& in, int B, int R, float* pred_logits, float
   if (!weights_loaded_) { *err = "lwdetr_forward: weights not loaded"; return -1; }
   if (B <= 0) { *err = "lwdetr_forward: batch must be positive"; return -1; }
   if ((B != planned_B_ || R != planned_R_) && plan(B, R, err)) return -1;
-  if (!in.images) { *err = "lwdetr_forward: null images"; return -1; }
+  if (in.kind == IN_U8_FRAMES ? !in.frames : !in.images) { *err = "lwdetr_forward: null images"; return -1; }
   in_ = in; in_topk_override_ = topk_override;
+  // the input op's byte count follows the input: a frames batch reads the frames, whatever their sizes
+  Op& gather = ops_[patch_op_];
+  gather.bytes = patch_bytes_;
+  if (in.kind == IN_U8_FRAMES) {
+    frames_.assign(in.frames, in.frames + B);
+    in_.frames = frames_.data();
+    gather.bytes = 2.0 * gather.rows * gather.cols;
+    for (const lwdetr_frame& f : frames_) gather.bytes += 3.0 * f.height * f.width;
+  }
   // The first forward of a plan always runs eagerly (it also performs the one-time cudaFuncSetAttribute calls).
   const bool graph_ok = use_graph_ && captures_.empty() && eager_runs_ > 0;
   if (graph_ok) {

@@ -36,13 +36,14 @@ struct Op {
   bool reads_input = false;   // consumes caller-owned pointers (images, mask): launched eagerly, never captured in the graph
 };
 
-// One forward's input: the image batch in one of three encodings plus the optional NestedTensor padding mask.
-enum : int { IN_F32_NCHW = 0, IN_16_NCHW = 1, IN_U8_NHWC = 2 };
+// One forward's input: the image batch in one of four encodings plus the optional NestedTensor padding mask.
+enum : int { IN_F32_NCHW = 0, IN_16_NCHW = 1, IN_U8_NHWC = 2, IN_U8_FRAMES = 3 };
 struct ForwardIn {
   const void* images = nullptr;   // DEVICE [B,3,R,R] fp32 / compute dtype, or [B,R,R,3] uint8
   int kind = IN_F32_NCHW;
+  const lwdetr_frame* frames = nullptr;   // IN_U8_FRAMES: HOST [B] descriptors of uint8 frames of any size (resized to R)
   const uint8_t* mask = nullptr;  // DEVICE bool [B,R,R] (True = padded pixel) or null
-  float mean[3] = {0.f, 0.f, 0.f}, stdv[3] = {1.f, 1.f, 1.f};   // IN_U8_NHWC: (x/255 - mean) / std
+  float mean[3] = {0.f, 0.f, 0.f}, stdv[3] = {1.f, 1.f, 1.f};   // IN_U8_NHWC / IN_U8_FRAMES: (x/255 - mean) / std
 };
 
 class Engine {
@@ -112,6 +113,9 @@ class Engine {
   std::vector<uint8_t> invalid_rows_;   // per memory token
   // live I/O pointers patched into the schedule at forward() time
   ForwardIn in_;
+  std::vector<lwdetr_frame> frames_;   // IN_U8_FRAMES: the last forward's descriptors (profile_ops re-runs them)
+  int patch_op_ = -1;                  // index of the input-reading "patch_gather" op in ops_
+  double patch_bytes_ = 0;             // its bytes for a [B,3,R,R] input; a frames forward reports the frames' bytes
   const int32_t* in_topk_override_ = nullptr;
   // result buffers (engine owned)
   float* out_logits_ = nullptr;   // [layers, B, nq, ldc_]

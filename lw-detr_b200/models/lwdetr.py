@@ -137,6 +137,27 @@ class LWDETR(nn.Module):
         out = self.engine().forward(x, want_aux=True, mask=mask)
         return self._pack_outputs(out)
 
+    @torch.no_grad()
+    def forward_frames(self, frames, img_size=None):
+        """frames: uint8 RGB frames of any size, as a decoder or camera delivers them - a [B, H, W, 3] tensor or a list of
+        [H_i, W_i, 3] tensors (host tensors are moved to the model's device).  Each frame is resized to img_size x
+        img_size (default cfg.img_size) on the device, bit-identical to the reference's host pre-processing
+        (demo.py:146-159: transforms.Resize([R, R]) on a PIL image, ToTensor, Normalize), so the outputs equal
+        forward() on those pre-processed images.  Boxes are normalised to each frame: PostProcess with target_sizes
+        (H_i, W_i) gives them in source pixels."""
+        if self.training:
+            raise RuntimeError("lwdetr_b200 implements the inference forward only; call model.eval()")
+        dev = next(self.parameters()).device
+        if dev.type != "cuda":
+            raise RuntimeError("lwdetr_b200: move the model to a CUDA device (no CPU fallback)")
+        R = self.cfg.img_size if img_size is None else int(img_size)
+        self._check_export_size(R)
+        if isinstance(frames, torch.Tensor):
+            frames = frames.to(dev)
+        else:
+            frames = [f.to(dev) if isinstance(f, torch.Tensor) else f for f in frames]
+        return self._pack_outputs(self.engine().forward_frames(frames, img_size=R, want_aux=True))
+
     def _check_export_size(self, R):
         # the reference's forward_export adds pos_embed_export, computed once for the 40x40 grid (vit.py:328-332)
         if self._export and R != self.cfg.img_size:
